@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA kernels via the C ABI)
   python bench.py --impl reference ...                      reference arm: the reference's OpenCV
                                                             CPU ops on the box's host cores
+  python bench.py ... --dump-outputs DIR                    our arm, and after the timed steps the
+                                                            outputs of the last one as DIR/<name>.npy
 
 Headline workload (config.workload): C3 -- 1080p Farneback OpticalFlow + FlowHistogram on ONE seeded
 synthetic clip of N*pairs+1 frames, frame-range sharded over the N ranks (sharding.pair_range: rank r
@@ -48,6 +50,29 @@ C5_BYTES = 343008000 + 8 * 1280 * 720 + 512 + 2764992   # 720p flow + flow histo
 C3_SEED, C4_SEED = 1000, 77
 C4_FRAMES = 32                      # 4K frames per rank and step (796 MB > L2)
 C5_STREAMS, C5_BATCH = 8, 16        # streams per GPU (64 streams on 8 GPUs), frames per stream per step
+
+# --dump-outputs: the flow histograms of every pair in full, the flow frames (1080p x 8 bytes each) as a
+# fixed seeded sample of pixels, the same for every pair, so that all files together stay within 64 MB
+DUMP_MAX_BYTES = 64 << 20
+DUMP_FLOW_BYTES = 48 << 20
+DUMP_SEED = 2024
+
+
+def dump_pixels(n_px, n_pairs):
+    """Sorted flat pixel indices (into H x W) of the flow sample that --dump-outputs writes."""
+    k = max(1, min(n_px, DUMP_FLOW_BYTES // (n_pairs * 8)))
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n_px, size=k, replace=False))
+
+
+def write_dump(out_dir, arrays):
+    """One out_dir/<name>.npy per output: float32 stays float32, everything else (integer counts) is written as
+    float64, which holds them exactly."""
+    arrays = {k: np.ascontiguousarray(a, np.float32 if a.dtype == np.float32 else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, ('--dump-outputs', total)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def measured_peaks():
@@ -357,6 +382,9 @@ def run_ours(args):
     lib.stb_farneback_profile(of._h, 0)
     fh_dev = d_fh.cpu().numpy().copy()
     flow_seam = (d_flow[0].cpu().numpy().copy(), d_flow[P - 1].cpu().numpy().copy())
+    if args.dump_outputs:
+        pix = torch.from_numpy(dump_pixels(H * W, world * P)).cuda()
+        flow_sample = d_flow.view(P, H * W, 2)[:, pix].cpu().numpy()
     del d_flow
 
     # ---- e2e: host frames in (pinned), flow histograms out (pinned), through the host-buffer C ABI.
@@ -445,6 +473,10 @@ def run_ours(args):
     # ---- per-frame outputs concatenated on the host in frame order; rank 0 re-computes every pair
     # that touches a shard seam ALONE (its own handle, frames generated from the seed) and compares
     all_fh = sharding.gather_frame_outputs(fh_dev, world * P, rank, world)
+    if args.dump_outputs:
+        all_flow_sample = sharding.gather_frame_outputs(flow_sample, world * P, rank, world)
+        if rank == 0:
+            write_dump(args.dump_outputs, {'flow_hist': all_fh, 'flow_sample': all_flow_sample})
     shard_check = None
     if rank == 0:
         seams = sorted({q for r in range(1, world) for q in (r * P - 1, r * P)} | {0, world * P - 1})
@@ -701,11 +733,18 @@ def main():
     ap.add_argument('--no-extra', action='store_true')
     ap.add_argument('--no-cpu', action='store_true')
     ap.add_argument('--no-flow-frames', action='store_true', help='skip the e2e_flow_frames figure (2 GB of pinned memory)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed (flow histograms of every pair, a fixed '
+                         'seeded sample of the flow frames) as DIR/<name>.npy, float32 or float64, at most 64 MB')
     ap.add_argument('--cpu-baseline-child', action='store_true', help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.cpu_baseline_child:
         cpu_baseline_child()
         return
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of our arm (--impl ours)')
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == 'reference':

@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -14,10 +15,26 @@ def pytest_configure(config):
     config.addinivalue_line('markers', 'gpu: needs a CUDA device (run on the B200 box with -m gpu)')
 
 
+class GoldenArrays(dict):
+    """The arrays of one fixture, read from `<stem>.npz` and its parts `<stem>.<k>.npz`
+    (tests/golden/make_golden.py splits a fixture so that no file exceeds 1 MB)."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
 @pytest.fixture(scope='session')
 def golden():
     def load(name):
-        return np.load(os.path.join(GOLDEN, name), allow_pickle=False)
+        stem = os.path.join(GOLDEN, name[:-len('.npz')])
+        out = GoldenArrays()
+        for path in [stem + '.npz'] + sorted(glob.glob(glob.escape(stem) + '.[0-9]*.npz')):
+            with np.load(path, allow_pickle=False) as z:
+                for k in z.files:
+                    assert k not in out, (path, k)
+                    out[k] = z[k]
+        return out
     return load
 
 

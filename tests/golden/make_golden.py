@@ -3,8 +3,10 @@ i.e. from OpenCV itself -- the library the reference's wrappers call.
 
 Run from the repo root:  python tests/golden/make_golden.py
 Inputs are stored alongside outputs (not only seeds) so the fixtures do not depend on the
-generator's numpy/cv2 versions when they are replayed.
+generator's numpy/cv2 versions when they are replayed.  shot_reference.npz is rewritten only when
+SCANNERTOOLS_REFERENCE names a checkout of the reference (ref_import.py).
 """
+import glob
 import os
 import sys
 import numpy as np
@@ -16,6 +18,28 @@ from oracle import cv2_ops  # noqa: E402
 from scannertools_b200 import synth  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+MAX_FILE_BYTES = 1000000
+PART_ARRAY_BYTES = 960000     # raw array bytes per file, leaving room for the npz container
+
+
+def save(name, **arrays):
+    """np.savez_compressed of the arrays into `<name>.npz`, continued in `<name>.1.npz`, `<name>.2.npz`, ...
+    where one file would pass MAX_FILE_BYTES; tests/conftest.py's `golden` fixture reads the parts as one."""
+    stem = os.path.join(HERE, name)
+    for old in glob.glob(glob.escape(stem) + '.[0-9]*.npz'):
+        os.remove(old)
+    parts, size = [{}], 0
+    for k, a in arrays.items():
+        nbytes = np.asarray(a).nbytes
+        if parts[-1] and size + nbytes > PART_ARRAY_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = a
+        size += nbytes
+    for i, part in enumerate(parts):
+        path = stem + ('.%d.npz' % i if i else '.npz')
+        np.savez_compressed(path, **part)
+        assert os.path.getsize(path) <= MAX_FILE_BYTES, (path, os.path.getsize(path))
 
 
 def make_resize_taps():
@@ -36,7 +60,7 @@ def make_resize_taps():
                 rs['out_%s_%s' % (interp, name)] = cv2.resize(img, (dw, dh), interpolation=getattr(cv2, interp))
     finally:
         cv2.ipp.setUseIPP(ipp0)
-    np.savez_compressed(os.path.join(HERE, 'resize_taps.npz'), meta=str(meta), **rs)
+    save('resize_taps', meta=str(meta), **rs)
 
 
 def main():
@@ -50,9 +74,9 @@ def main():
     clip, cuts = synth.cut_clip(5, 1000, 360, 640, n_cuts=7)
     hists = np.stack([cv2_ops.histogram(f) for f in clip]).astype(np.int32)
     bounds = cv2_ops.shot_boundaries(list(hists))
-    np.savez_compressed(os.path.join(HERE, 'shot_c1.npz'), hists=hists, boundaries=np.array(bounds, np.int32),
-                        cuts=np.array(cuts, np.int32), scores=cv2_ops.shot_scores(hists),
-                        frame0=clip[0], frame_first_cut=clip[cuts[0]], meta=str(meta))
+    save('shot_c1', hists=hists, boundaries=np.array(bounds, np.int32),
+         cuts=np.array(cuts, np.int32), scores=cv2_ops.shot_scores(hists),
+         frame0=clip[0], frame_first_cut=clip[cuts[0]], meta=str(meta))
     print('shot_c1: boundaries', bounds, 'cuts', cuts)
 
     # small histogram cases incl. ragged widths (rows not 4/16-byte aligned) and constants
@@ -64,7 +88,7 @@ def main():
                      ('one_px', synth.noise_clip(13, 1, 1, 1)[0])]:
         hs['in_' + name] = fr
         hs['out_' + name] = cv2_ops.histogram(fr)
-    np.savez_compressed(os.path.join(HERE, 'hist_small.npz'), meta=str(meta), **hs)
+    save('hist_small', meta=str(meta), **hs)
 
     # Farneback: textured pairs at sizes covering 4 scales, 3 scales, and round-half-even
     fl = {}
@@ -74,7 +98,7 @@ def main():
         fl['f1_' + name] = c[1]
         fl['gray0_' + name] = cv2_ops.gray(c[0])
         fl['flow_' + name] = cv2_ops.optical_flow(c[0], c[1])
-    np.savez_compressed(os.path.join(HERE, 'flow_small.npz'), meta=str(meta), **fl)
+    save('flow_small', meta=str(meta), **fl)
 
     # FlowHistogram: a real flow field and the stress field
     fh = {}
@@ -89,12 +113,12 @@ def main():
         if f.size < 4096:
             fh['mag_' + name] = mag
             fh['deg_' + name] = deg
-    np.savez_compressed(os.path.join(HERE, 'flowhist.npz'), meta=str(meta), **fh)
+    save('flowhist', meta=str(meta), **fh)
 
     # FrameDifference (intended semantics)
     a = synth.noise_clip(21, 2, 19, 23)
-    np.savez_compressed(os.path.join(HERE, 'framediff.npz'), prev=a[0], cur=a[1],
-                        out=cv2_ops.frame_difference(a[0], a[1]), meta=str(meta))
+    save('framediff', prev=a[0], cur=a[1],
+         out=cv2_ops.frame_difference(a[0], a[1]), meta=str(meta))
     # Resize (next row): down-scale to the shipped pipeline's 426x240, exact 2x, up-scale, gray
     rs = {}
     rng = np.random.default_rng(31)
@@ -103,7 +127,7 @@ def main():
         img = rng.integers(0, 256, (sh, sw, cn) if cn > 1 else (sh, sw), dtype=np.uint8)
         rs['in_' + name] = img
         rs['out_' + name] = cv2_ops.resize(img, dw, dh)
-    np.savez_compressed(os.path.join(HERE, 'resize.npz'), meta=str(meta), **rs)
+    save('resize', meta=str(meta), **rs)
     # ConvertColor (next row): the conversions the B200 build implements
     rng = np.random.default_rng(77)
     img = rng.integers(0, 256, (60, 107, 3), dtype=np.uint8)
@@ -111,9 +135,9 @@ def main():
     cc = {'in': img}
     for name in ['COLOR_RGB2HSV', 'COLOR_BGR2HSV', 'COLOR_RGB2GRAY', 'COLOR_BGR2GRAY', 'COLOR_RGB2BGR']:
         cc[name] = cv2_ops.convert_color(img, name)
-    np.savez_compressed(os.path.join(HERE, 'convert_color.npz'), meta=str(meta), **cc)
-    # ShotBoundaries goldens from the REFERENCE ITSELF (its Python op imported from /root/reference
-    # behind a scannerpy stub, ref_import.py): histogram sequences -> boundary lists
+    save('convert_color', meta=str(meta), **cc)
+    # ShotBoundaries goldens from the REFERENCE ITSELF (its Python op imported from the checkout that
+    # SCANNERTOOLS_REFERENCE names, behind a scannerpy stub, ref_import.py): histogram sequences -> boundary lists
     import ref_import
     if ref_import.available():
         sd, ty = ref_import.load('shot_detection'), ref_import.load('types')
@@ -132,8 +156,7 @@ def main():
             rows = sd.shot_boundaries(None, [ty.histograms(x.tobytes(), None) for x in h])
             cases['hist_' + name] = h
             cases['bounds_' + name] = np.array(rows[0], np.int32)
-        np.savez_compressed(os.path.join(HERE, 'shot_reference.npz'),
-                            meta='generated by the reference scannertools/shot_detection.py::shot_boundaries', **cases)
+        save('shot_reference', meta='generated by the reference scannertools/shot_detection.py::shot_boundaries', **cases)
     for f in sorted(os.listdir(HERE)):
         if f.endswith('.npz'):
             print(f, os.path.getsize(os.path.join(HERE, f)))

@@ -1,21 +1,21 @@
-"""Imports the reference's own Python code for this path from /root/reference (available only in
-the build container, never on the GPU box) behind a minimal stub of `scannerpy`, so that goldens
-can be produced by the REFERENCE ITSELF where it is Python:
+"""Imports the reference's own Python code for this path from a checkout of the reference
+(scanner-research/scannertools) named by the environment variable SCANNERTOOLS_REFERENCE, behind a
+minimal stub of `scannerpy`, so that goldens can be produced by the REFERENCE ITSELF where it is Python:
 
   * scannertools/shot_detection.py   -> shot_boundaries(config, histograms)
   * scannertools/types.py            -> histograms(buf, protobufs)
 
-Used by make_golden.py and by tests/test_oracle.py (skipped when /root/reference is absent)."""
+Used by make_golden.py only; the tests replay what it wrote (shot_reference.npz)."""
 import importlib.util
 import os
 import sys
 import types
 
-REF = '/root/reference/scannertools/scannertools'
+REF = os.path.join(os.environ['SCANNERTOOLS_REFERENCE'], 'scannertools') if os.environ.get('SCANNERTOOLS_REFERENCE') else None
 
 
 def available():
-    return os.path.isfile(os.path.join(REF, 'shot_detection.py'))
+    return REF is not None and os.path.isfile(os.path.join(REF, 'shot_detection.py'))
 
 
 def _stub_scannerpy():

@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), '..'))
 from scannertools_b200 import ops
 def timeit(fn, iters=20, warm=3):
     for _ in range(warm): fn()
