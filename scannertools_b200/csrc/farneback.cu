@@ -964,14 +964,27 @@ __device__ __forceinline__ void update_matrices_px(const float* __restrict__ R0,
                     __ldg(R0 + 4 * n + o), R1, n, w, h, x, y, dx, dy, m);
 }
 
+// Flow-compensated R1 window of iter15_win_kernel: the box [x0, x0 + kWinW) x [y0, y0 + kWinH) of the
+// five R1 planes in shared memory, plane stride kWinPlaneFloats.  fits == false: no window, the
+// footprints are gathered from global memory (kNoR1Win, a compile-time constant for the other kernels).
+constexpr int kWinW = 56, kWinH = 38;
+constexpr int kWinPlaneFloats = 2144;                         // 56 * 38 = 2128, rounded up to a multiple of 32 floats (128 B)
+struct R1Win {
+  const float* s;
+  int x0, y0;
+  bool fits;
+};
+constexpr R1Win kNoR1Win = {nullptr, 0, 0, false};
+
 // Two VERTICALLY adjacent pixels (x, y) and (x, y+1) handled by one thread, consecutive lanes on
 // consecutive x.  Their bilinear footprints in R1 almost always share a row (floor(y + dy) of
 // vertical neighbours differs by exactly 1 except at integer crossings), so 3 rows x 2 columns
 // per plane serve both pixels (30 loads instead of 40), and -- unlike a horizontal pair, whose
 // lanes stride by two pixels -- every load of a warp covers one contiguous run of floats: about
 // 1.3 L1 wavefronts per load instead of 3.  Same values and arithmetic as two single calls.
-__device__ __forceinline__ void update_matrices_vpair(const float* __restrict__ R0, const float* __restrict__ R1, int n,
-                                                      int w, int h, int x, int y, float2 fa, float2 fb, float ma[5],
+// With a window that fits, the shared footprint is read from it instead (same values).
+__device__ __forceinline__ void update_matrices_vpair(const float* __restrict__ R0, const float* __restrict__ R1, R1Win win,
+                                                      int n, int w, int h, int x, int y, float2 fa, float2 fb, float ma[5],
                                                       float mb[5]) {
   float qa[5], qb[5];
   {
@@ -989,18 +1002,30 @@ __device__ __forceinline__ void update_matrices_vpair(const float* __restrict__ 
     fxa -= (float)x1a; fya -= (float)y1a; fxb -= (float)x1b; fyb -= (float)y1b;
     const float a00 = (1.f - fxa) * (1.f - fya), a01 = fxa * (1.f - fya), a10 = (1.f - fxa) * fya, a11 = fxa * fya;
     const float b00 = (1.f - fxb) * (1.f - fyb), b01 = fxb * (1.f - fyb), b10 = (1.f - fxb) * fyb, b11 = fxb * fyb;
-    const float* p = padd(R1, y1a * w + x1a);
     float ra[5], rb[5];
+    if (win.fits) {
+      const float* p = win.s + (y1a - win.y0) * kWinW + (x1a - win.x0);
 #pragma unroll
-    for (int pl = 0; pl < 5; ++pl) {
-      const float* p1 = padd(p, w);
-      const float* p2 = padd(p1, w);
-      const float t00 = __ldg(p), t01 = __ldg(p + 1);
-      const float t10 = __ldg(p1), t11 = __ldg(p1 + 1);
-      const float t20 = __ldg(p2), t21 = __ldg(p2 + 1);
-      ra[pl] = a00 * t00 + a01 * t01 + a10 * t10 + a11 * t11;
-      rb[pl] = b00 * t10 + b01 * t11 + b10 * t20 + b11 * t21;
-      p = padd(p, n);
+      for (int pl = 0; pl < 5; ++pl) {
+        const float t00 = p[pl * kWinPlaneFloats], t01 = p[pl * kWinPlaneFloats + 1];
+        const float t10 = p[pl * kWinPlaneFloats + kWinW], t11 = p[pl * kWinPlaneFloats + kWinW + 1];
+        const float t20 = p[pl * kWinPlaneFloats + 2 * kWinW], t21 = p[pl * kWinPlaneFloats + 2 * kWinW + 1];
+        ra[pl] = a00 * t00 + a01 * t01 + a10 * t10 + a11 * t11;
+        rb[pl] = b00 * t10 + b01 * t11 + b10 * t20 + b11 * t21;
+      }
+    } else {
+      const float* p = padd(R1, y1a * w + x1a);
+#pragma unroll
+      for (int pl = 0; pl < 5; ++pl) {
+        const float* p1 = padd(p, w);
+        const float* p2 = padd(p1, w);
+        const float t00 = __ldg(p), t01 = __ldg(p + 1);
+        const float t10 = __ldg(p1), t11 = __ldg(p1 + 1);
+        const float t20 = __ldg(p2), t21 = __ldg(p2 + 1);
+        ra[pl] = a00 * t00 + a01 * t01 + a10 * t10 + a11 * t11;
+        rb[pl] = b00 * t10 + b01 * t11 + b10 * t20 + b11 * t21;
+        p = padd(p, n);
+      }
     }
     um_finish(qa[0], qa[1], qa[2], qa[3], qa[4], true, ra[0], ra[1], ra[2], ra[3], ra[4], w, h, x, y, fa.x, fa.y, ma);
     um_finish(qb[0], qb[1], qb[2], qb[3], qb[4], true, rb[0], rb[1], rb[2], rb[3], rb[4], w, h, x, y + 1, fb.x, fb.y, mb);
@@ -1011,62 +1036,40 @@ __device__ __forceinline__ void update_matrices_vpair(const float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Block order of the kernels that read R (updmat_init_kernel and the iteration kernels): a 1-D grid
-// walked PAIR-FASTEST.  The polynomial expansion R of frame f+1 is read twice per level and pass:
+// Block order of the kernels that read R (updmat_init_kernel and the iteration kernels): the grid
+// is walked PAIR-FASTEST.  The polynomial expansion R of frame f+1 is read twice per level and pass:
 // displaced, as R1 of pair f, and in place, as R0 of pair f+1.  With the pair index as the slowest
 // grid dimension (round 1) those two reads were a whole pair (2.3 resident waves, ~200 MB of
 // traffic) apart and both came from HBM; with the pairs of one tile adjacent in the grid they run
 // at the same time on neighbouring SMs and the second read is an L2 hit: a quarter of the
-// iteration's 80 B/px never reaches HBM.  Order: pair, then `band` tile rows, then tile column,
-// then band, so a tile's vertical neighbours (whose M halos it shares) are co-resident too.
+// iteration's 80 B/px never reaches HBM.  Two orders are launched:
+//   * the iteration kernels: a 1-D grid, pair, then kTileBand tile rows, then tile column, then
+//     band, so a tile's vertical neighbours (whose M halos it shares) are co-resident too;
+//   * updmat_init_kernel: a 3-D grid (pair, tile x, tile y) in the hardware's own rasterisation
+//     order.
+// Measured on B200 (1080p, 16-pair batches, one box, back to back): round-1 order through a 1-D grid
+// 5117 fps; iteration kernels band 2 / 4 / 8 / all rows: 5284 / 5308 / 5317 / 5001; updmat_init_kernel
+// band 8 / 16 / 32 / all rows: 5309 / 5308 / 5314 / 5193 and, as the 3-D grid: +1.5 % on top (5466 vs
+// 5383) -- the iteration kernels lose 0.4 % that way.
 // ---------------------------------------------------------------------------------------------
+constexpr int kTileBand = 4;   // tile rows of 32 px walked before the column advances
+
 struct TileOrder {
-  int tiles_x, tiles_y, np, band;     // band = tile rows walked before the column advances; 0 = round-1 order (x, y, pair);
-                                      // < 0 = 3-D grid (pair, tile x, tile y)
+  int tiles_x, tiles_y, np;
 };
 
-__device__ __forceinline__ void tile_decode(const TileOrder& o, int id, int& tx, int& ty, int& pz) {
-  if (o.band == -2) {  // round-1 launch shape: 3-D grid (tile x, tile y, pair)
-    const int per = o.tiles_x * o.tiles_y;
-    pz = id / per;
-    const int r = id - pz * per;
-    ty = r / o.tiles_x;
-    tx = r - ty * o.tiles_x;
-    return;
-  }
-  if (o.band < 0) {   // 3-D grid (pair, tile x, tile y) in the hardware's own rasterisation order
-    const int per = o.np * o.tiles_x;
-    ty = id / per;
-    const int r = id - ty * per;
-    tx = r / o.np;
-    pz = r - tx * o.np;
-    return;
-  }
-  if (o.band <= 0) {
-    const int per = o.tiles_x * o.tiles_y;
-    pz = id / per;
-    const int r = id - pz * per;
-    ty = r / o.tiles_x;
-    tx = r - ty * o.tiles_x;
-    return;
-  }
-  const int per_band = o.tiles_x * o.band * o.np;
-  const int b = id / per_band, r = id - b * per_band;
-  const int bh = min(o.band, o.tiles_y - b * o.band);      // the last band may be shorter
-  const int col = bh * o.np;
-  tx = r / col;
-  const int r2 = r - tx * col;
-  const int tyb = r2 / o.np;
-  ty = b * o.band + tyb;
-  pz = r2 - tyb * o.np;
-}
-
-// this block's tile: 3-D grids map blockIdx directly (no integer division)
-__device__ __forceinline__ void tile_of_block(const TileOrder& o, int& tx, int& ty, int& pz, int& bid) {
-  bid = (int)(blockIdx.x + gridDim.x * (blockIdx.y + gridDim.y * blockIdx.z));
-  if (o.band == -1) { pz = (int)blockIdx.x; tx = (int)blockIdx.y; ty = (int)blockIdx.z; }
-  else if (o.band == -2) { tx = (int)blockIdx.x; ty = (int)blockIdx.y; pz = (int)blockIdx.z; }
-  else tile_decode(o, bid, tx, ty, pz);
+// tile of block `id` of the iteration kernels' 1-D grid.  Unsigned divisions: shorter than signed
+// ones, which keeps the 64-register kernels free of spills.
+__device__ __forceinline__ void tile_of_band_order(const TileOrder& o, int id, int& tx, int& ty, int& pz) {
+  const unsigned per_band = (unsigned)(o.tiles_x * kTileBand * o.np);
+  const unsigned b = (unsigned)id / per_band, r = (unsigned)id - b * per_band;
+  const unsigned bh = min((unsigned)kTileBand, (unsigned)o.tiles_y - b * kTileBand);   // the last band may be shorter
+  const unsigned col = bh * (unsigned)o.np;
+  tx = (int)(r / col);
+  const unsigned r2 = r - (unsigned)tx * col;
+  const unsigned tyb = r2 / (unsigned)o.np;
+  ty = (int)(b * kTileBand + tyb);
+  pz = (int)(r2 - tyb * (unsigned)o.np);
 }
 
 // initial M of a level from the up-sampled coarser flow (Appendix A.4-5).
@@ -1098,16 +1101,14 @@ __device__ __forceinline__ float2 upsample_flow(const float2* __restrict__ fc, i
 // Two horizontally adjacent pixels per thread (8-byte accesses of R0 / M when w is even).  This
 // kernel is DRAM-bound (69 % of peak): the vertical-pair mapping that helps the L1-bound iteration
 // kernel measured 12 % slower here (495 vs 440 us per 16-pair level-0 launch).
-// 5 blocks/SM (48 registers, no spills): with the prefetch-ahead in place the extra resident warps are
+// 5 blocks/SM (48 registers): with the prefetch-ahead in place the extra resident warps are
 // worth +1 % of the step (before it, 5 blocks/SM measured slower: 500 vs 440 us in isolation).
-template <int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// Grid (pair, tile x, tile y) of 64 x 8 tiles, see "Block order" above.
+__global__ void __launch_bounds__(256, 5)
 updmat_init_kernel(const float* __restrict__ R, const float* __restrict__ flow_coarse, float* __restrict__ M,
                    int w, int h, int wc, int hc, double scale_x, double scale_y, float flow_mul, int pair0,
-                   const STB_GRID_CONSTANT TmaMap3D map_R, int prefetch_blocks, TileOrder ord) {
-  int btx, bty, bpz;
-  int bid;
-  tile_of_block(ord, btx, bty, bpz, bid);
+                   const STB_GRID_CONSTANT TmaMap3D map_R, int prefetch_blocks) {
+  const int bpz = (int)blockIdx.x, btx = (int)blockIdx.y, bty = (int)blockIdx.z;
   const int pair = pair0 + bpz;
   if (prefetch_blocks > 0 && threadIdx.x < 10) {
     // The block `prefetch_blocks` further on in the grid is picked up about two resident waves from
@@ -1115,11 +1116,12 @@ updmat_init_kernel(const float* __restrict__ R, const float* __restrict__ flow_c
     // of every frame tile is prefetched by exactly one block: a block prefetches R0 (the planes of its
     // own frame, lanes 0-4); the block of the launch's last pair also prefetches R1 (lanes 5-9) -- for
     // the other pairs that frame is the R0 of the pair next to them.
-    const int ahead = bid + prefetch_blocks;
+    const int np = (int)gridDim.x, per = np * (int)gridDim.y;
+    const int ahead = (int)(blockIdx.x + gridDim.x * (blockIdx.y + gridDim.y * blockIdx.z)) + prefetch_blocks;
     if (ahead < (int)(gridDim.x * gridDim.y * gridDim.z)) {
-      int atx, aty, apz;
-      tile_decode(ord, ahead, atx, aty, apz);
-      if ((int)threadIdx.x < 5 || ord.band == 0 || ord.band == -2 || apz == ord.np - 1)
+      const int aty = ahead / per, r = ahead - aty * per;
+      const int atx = r / np, apz = r - atx * np;
+      if ((int)threadIdx.x < 5 || apz == np - 1)
         tma_prefetch_l2(&map_R, atx * 64, aty * 8, (pair0 + apz) * 5 + (int)threadIdx.x);
     }
   }
@@ -1374,10 +1376,11 @@ constexpr int kFiFlStride = kFiTW + 1;        // float2 row stride of the staged
 //           (update_matrices_vpair): unit-stride R1 gathers with a shared middle row.  Measured on
 //           B200 against the alternatives: one pixel per thread 618 us, two horizontally adjacent
 //           pixels with 8-byte R0 / M' accesses 555 us per 16-pair level-0 launch.
+//           R1 footprints come from `win` when it fits (iter15_win_kernel).
 //   !UPDATE: two horizontally adjacent pixels per thread so the flow goes out as 16-byte stores.
 template <bool UPDATE, bool HIST>
 __device__ __forceinline__ void iter15_global_phase(const float2* fl, unsigned* fh, float* __restrict__ Mout,
-                                                    const float* __restrict__ R, const PtrBatch<float>& flow_out,
+                                                    const float* __restrict__ R, R1Win win, const PtrBatch<float>& flow_out,
                                                     int32_t* __restrict__ flow_hist, int w, int h, int pair, int pz, int ox0, int oy0) {
   const int tid = threadIdx.x, warp = tid >> 5;
   const size_t n = (size_t)w * h;
@@ -1397,7 +1400,7 @@ __device__ __forceinline__ void iter15_global_phase(const float2* fl, unsigned* 
       float* Mo = Mp + (y * w + x);
       float ma[5], mb[5];
       if (y + 1 < h) {
-        update_matrices_vpair(R0, R1, ni, w, h, x, y, fa, fb, ma, mb);
+        update_matrices_vpair(R0, R1, win, ni, w, h, x, y, fa, fb, ma, mb);
 #pragma unroll
         for (int c = 0; c < 5; ++c) { *Mo = ma[c]; *padd(Mo, w) = mb[c]; Mo = padd(Mo, ni); }
       } else {
@@ -1477,6 +1480,24 @@ __device__ __forceinline__ float2 solve_flow15(float g11, float g12, float g22, 
   return make_float2(nx * idet, ny * idet);
 }
 
+// Horizontal pass of one plane over its transposed vertical sums vt: lane = output row, warp = group
+// of kFiGC output columns.
+__device__ __forceinline__ void box15_rows(const float* vt, float out[kFiGC]) {
+  const float* rowp = vt + ((threadIdx.x >> 5) * kFiGC) * 33 + (threadIdx.x & 31);
+  float t[kFiGC + 14];
+#pragma unroll
+  for (int j = 0; j < kFiGC + 14; ++j) t[j] = rowp[j * 33];
+  box15<kFiGC>(t, out);
+}
+
+// Flow of this thread's output i (row lane, column warp * kFiGC + i) from the window sums, staged in
+// fl for the global phase.
+__device__ __forceinline__ float2 stage_flow15(float2* fl, const float (&sums)[5][kFiGC], int i) {
+  const float2 f = solve_flow15(sums[0][i], sums[1][i], sums[2][i], sums[3][i], sums[4][i]);
+  fl[(threadIdx.x & 31) * kFiFlStride + (threadIdx.x >> 5) * kFiGC + i] = f;
+  return f;
+}
+
 template <bool UPDATE, bool HIST>
 __global__ void __launch_bounds__(kFiThreads, 4)
 iter15_kernel(const float* __restrict__ Min, float* __restrict__ Mout, const float* __restrict__ R,
@@ -1488,10 +1509,9 @@ iter15_kernel(const float* __restrict__ Min, float* __restrict__ Mout, const flo
     for (int i = threadIdx.x; i < (kFiThreads / 32) * kFiHistStride; i += kFiThreads) fh[i] = 0u;
   }
 
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int tid = threadIdx.x;
   int btx, bty, bpz;
-  int bid;
-  tile_of_block(ord, btx, bty, bpz, bid);
+  tile_of_band_order(ord, (int)blockIdx.x, btx, bty, bpz);
   const int pair = pair0 + bpz;
   const size_t n = (size_t)w * h;
   const float* Mp = Min + (size_t)pair * 5 * n;
@@ -1535,22 +1555,15 @@ iter15_kernel(const float* __restrict__ Min, float* __restrict__ Mout, const flo
       if (c < 4) load_plane(c + 1);   // in flight across the barrier and the horizontal pass
     }
     __syncthreads();
-    {
-      const float* rowp = vt + (warp * kFiGC) * 33 + lane;
-      float t[kFiGC + 14];
-#pragma unroll
-      for (int j = 0; j < kFiGC + 14; ++j) t[j] = rowp[j * 33];
-      box15<kFiGC>(t, sums[c]);
-    }
+    box15_rows(vt, sums[c]);
     // Vt[c&1] is next written for plane c+2, after the barrier of plane c+1: safe.
   }
 
 #pragma unroll
-  for (int i = 0; i < kFiGC; ++i)
-    fl[lane * kFiFlStride + warp * kFiGC + i] = solve_flow15(sums[0][i], sums[1][i], sums[2][i], sums[3][i], sums[4][i]);
+  for (int i = 0; i < kFiGC; ++i) stage_flow15(fl, sums, i);
   __syncthreads();
 
-  iter15_global_phase<UPDATE, HIST>(fl, fh, Mout, R, flow_out, flow_hist, w, h, pair, bpz, ox0, oy0);
+  iter15_global_phase<UPDATE, HIST>(fl, fh, Mout, R, kNoR1Win, flow_out, flow_hist, w, h, pair, bpz, ox0, oy0);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1622,53 +1635,42 @@ __device__ __forceinline__ void tma_load_tile(float* dst, const TmaMap3D* map, i
 }
 #endif
 
-template <bool UPDATE, bool HIST>
-__global__ void __launch_bounds__(kFiThreads, 4)
-iter15_tma_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ Mout, const float* __restrict__ R,
-                  PtrBatch<float> flow_out, int32_t* __restrict__ flow_hist, int w, int h, int pair0,
-                  const STB_GRID_CONSTANT TmaMap3D map_R, int prefetch_R, TileOrder ord) {
-  __shared__ __align__(128) float raw[2][kTmStageFloats];     // also reused for the staged flow after the box phase
-  __shared__ float Vt[2][kFiVtWords];
-  __shared__ __align__(8) unsigned long long bars[2];
-  __shared__ unsigned fh[HIST ? (kFiThreads / 32) * kFiHistStride : 1];
-  float2* fl = reinterpret_cast<float2*>(&raw[0][0]);       // 32 x 49 float2 = 12544 B <= one stage + part of the next
-  static_assert(kFiTH * kFiFlStride * sizeof(float2) <= 2 * kTmStageBytes, "staged flow must fit in the raw ring");
+// Box phase of iter15_tma_kernel and iter15_win_kernel: initialises bars[0 .. NBARS) (the ones past the
+// two of the ring are the caller's), streams the tile's five M planes through the ring raw / bars[0..1],
+// and leaves the horizontal 15-sums of this thread's outputs in sums.  The shared buffers are passed in
+// because one kernel holds them as static arrays and the other in its dynamic overlay.  Ends with a
+// barrier after the last read of raw and Vt, so the caller may overlay them.
+template <int NBARS>
+__device__ __forceinline__ void iter15_tma_box(float (*raw)[kTmStageFloats], float (*Vt)[kFiVtWords], unsigned long long* bars,
+                                               const TmaMap3D* map_in, const TmaMap3D* map_R, bool prefetch_R, bool last_pair,
+                                               int w, int h, int pair, int ox0, int oy0, float (&sums)[5][kFiGC]) {
   static_assert(kFiRawW + 1 <= kTmRawW && (kFiTW % 4) == 0, "box covers the halo'd tile from an aligned origin");
-
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  int btx, bty, bpz;
-  int bid;
-  tile_of_block(ord, btx, bty, bpz, bid);
-  const int pair = pair0 + bpz;
-  const int ox0 = btx * kFiTW, oy0 = bty * kFiTH;
+  const int tid = threadIdx.x;
   // box origin (may be negative).  The innermost TMA coordinate must be 16-byte aligned (measured:
   // an unaligned x traps), so the box starts one column early: raw column cx lives at box column cx+1.
   const int bx0 = ox0 - kFiM - 1, by0 = oy0 - kFiM;
 
-  if (HIST) {
-    for (int i = tid; i < (kFiThreads / 32) * kFiHistStride; i += kFiThreads) fh[i] = 0u;
-  }
   if (tid == 0) {
-    tma_mbar_init(&bars[0], 1);
-    tma_mbar_init(&bars[1], 1);
+#pragma unroll
+    for (int b = 0; b < NBARS; ++b) tma_mbar_init(&bars[b], 1);
 #ifndef STB_CPU_EMU
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 #endif
   }
   __syncthreads();
   if (tid == 0) {
-    tma_load_tile(raw[0], &map_in, bx0, by0, pair * 5 + 0, &bars[0]);
-    tma_load_tile(raw[1], &map_in, bx0, by0, pair * 5 + 1, &bars[1]);
+    tma_load_tile(raw[0], map_in, bx0, by0, pair * 5 + 0, &bars[0]);
+    tma_load_tile(raw[1], map_in, bx0, by0, pair * 5 + 1, &bars[1]);
   }
   // (pair-fastest order: R1 of this pair is the R0 of the pair next to it, whose block runs at the same time and
   // prefetches it; only the launch's last pair has to pull its own R1)
-  if (UPDATE && prefetch_R && tid >= 32 && tid < ((ord.band == 0 || ord.band == -2 || bpz == ord.np - 1) ? 42 : 37)) {
+  if (prefetch_R && tid >= 32 && tid < (last_pair ? 42 : 37)) {
     // the update phase at the end of this block reads this tile of R0 (frame `pair`) and, displaced
     // by the flow, of R1 (frame pair + 1): pull both towards L2 while the box phase runs, so those
     // loads find L2 hits instead of paying DRAM latency on the critical path (543 -> 522 us per
     // 16-pair level-0 launch)
     const int q = tid - 32;                      // 0..4: R0 planes, 5..9: R1 planes
-    tma_prefetch_l2(&map_R, ox0, oy0, pair * 5 + q);
+    tma_prefetch_l2(map_R, ox0, oy0, pair * 5 + q);
   }
   // (Prefetching the M boxes of a tile one or two waves ahead, the way updmat_init_kernel does for
   // R, was measured and rejected: 599-628 us vs 533-542 us per 16-pair level-0 launch, with
@@ -1682,7 +1684,6 @@ iter15_tma_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ M
   const bool border = (bx0 + 1 < 0) || (by0 < 0) || (bx0 + 1 + kFiRawW > w) || (by0 + kTmRawH > h);
   const int ccol = min(max(bx0 + 1 + vcx, 0), w - 1) - bx0;  // clamped column inside the box
 
-  float sums[5][kFiGC];
 #pragma unroll
   for (int c = 0; c < 5; ++c) {
     const int st = c & 1;
@@ -1708,23 +1709,40 @@ iter15_tma_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ M
       for (int i = 0; i < 8; ++i) o[i] = vs[i];
     }
     __syncthreads();                                           // raw[st] consumed, Vt[st] complete
-    if (tid == 0 && c + 2 < 5) tma_load_tile(raw[st], &map_in, bx0, by0, pair * 5 + c + 2, &bars[st]);
-    {
-      const float* rowp = vt + (warp * kFiGC) * 33 + lane;
-      float t[kFiGC + 14];
-#pragma unroll
-      for (int j = 0; j < kFiGC + 14; ++j) t[j] = rowp[j * 33];
-      box15<kFiGC>(t, sums[c]);
-    }
+    if (tid == 0 && c + 2 < 5) tma_load_tile(raw[st], map_in, bx0, by0, pair * 5 + c + 2, &bars[st]);
+    box15_rows(vt, sums[c]);
   }
-  __syncthreads();   // every read of raw (plane 4 lives in stage 0) is done before fl aliases it
+  __syncthreads();   // every read of raw (plane 4 lives in stage 0) and Vt is done before the caller overlays them
+}
+
+template <bool UPDATE, bool HIST>
+__global__ void __launch_bounds__(kFiThreads, 4)
+iter15_tma_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ Mout, const float* __restrict__ R,
+                  PtrBatch<float> flow_out, int32_t* __restrict__ flow_hist, int w, int h, int pair0,
+                  const STB_GRID_CONSTANT TmaMap3D map_R, int prefetch_R, TileOrder ord) {
+  __shared__ __align__(128) float raw[2][kTmStageFloats];     // also reused for the staged flow after the box phase
+  __shared__ float Vt[2][kFiVtWords];
+  __shared__ __align__(8) unsigned long long bars[2];
+  __shared__ unsigned fh[HIST ? (kFiThreads / 32) * kFiHistStride : 1];
+  float2* fl = reinterpret_cast<float2*>(&raw[0][0]);       // 32 x 49 float2 = 12544 B <= one stage + part of the next
+  static_assert(kFiTH * kFiFlStride * sizeof(float2) <= 2 * kTmStageBytes, "staged flow must fit in the raw ring");
+
+  int btx, bty, bpz;
+  tile_of_band_order(ord, (int)blockIdx.x, btx, bty, bpz);
+  const int pair = pair0 + bpz;
+  const int ox0 = btx * kFiTW, oy0 = bty * kFiTH;
+
+  if (HIST) {
+    for (int i = threadIdx.x; i < (kFiThreads / 32) * kFiHistStride; i += kFiThreads) fh[i] = 0u;
+  }
+  float sums[5][kFiGC];
+  iter15_tma_box<2>(raw, Vt, bars, &map_in, &map_R, UPDATE && prefetch_R, bpz == ord.np - 1, w, h, pair, ox0, oy0, sums);
 
 #pragma unroll
-  for (int i = 0; i < kFiGC; ++i)
-    fl[lane * kFiFlStride + warp * kFiGC + i] = solve_flow15(sums[0][i], sums[1][i], sums[2][i], sums[3][i], sums[4][i]);
+  for (int i = 0; i < kFiGC; ++i) stage_flow15(fl, sums, i);
   __syncthreads();
 
-  iter15_global_phase<UPDATE, HIST>(fl, fh, Mout, R, flow_out, flow_hist, w, h, pair, bpz, ox0, oy0);
+  iter15_global_phase<UPDATE, HIST>(fl, fh, Mout, R, kNoR1Win, flow_out, flow_hist, w, h, pair, bpz, ox0, oy0);
 }
 
 
@@ -1741,70 +1759,17 @@ iter15_tma_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ M
 // issues their (flow-independent) R0 loads; the bilinear footprints are then LDS with immediate
 // offsets off one base address.  Smooth flow -- any global motion, however large -- fits; tiles
 // that straddle a motion boundary do not and take the global-memory gathers, as do pixel pairs
-// whose footprints do not share a row.  Same arithmetic as update_matrices_vpair.
+// whose footprints do not share a row.  Box phase and update loop are iter15_tma_kernel's
+// (iter15_tma_box, iter15_global_phase), the latter given the window.
 // Shared memory: raw ring + Vt (39.9 KB, dead after the box phase) are overlaid by the staged flow
 // (12.25 KB) and the window (5 x 8.4 KB): 55.5 KB per block, still 4 blocks per SM.
 // ---------------------------------------------------------------------------------------------
-constexpr int kWinW = 56, kWinH = 38;
-constexpr int kWinPlaneFloats = 2144;                         // 56 * 38 = 2128, rounded up to a multiple of 32 floats (128 B)
 constexpr size_t kWinFlBytes = 12544;                         // 32 x 49 float2
 constexpr size_t kWinSmemWin = kWinFlBytes;                   // window starts right after the staged flow
 constexpr size_t kWinSmemBars = kWinSmemWin + 5 * kWinPlaneFloats * sizeof(float);   // 55424
 constexpr size_t kWinSmemBytes = kWinSmemBars + 64;
 static_assert(kWinW * kWinH <= kWinPlaneFloats && (kWinFlBytes % 128) == 0 && ((kWinPlaneFloats * 4) % 128) == 0, "TMA destinations are 128-byte aligned");
 static_assert(2 * kTmStageBytes + 2 * kFiVtWords * sizeof(float) <= kWinSmemBars, "box-phase buffers fit under the barriers");
-
-__device__ __forceinline__ void um_vpair_win(const float* __restrict__ R0, const float* __restrict__ R1, const float* __restrict__ win,
-                                             int wx0, int wy0, bool fits, int n, int w, int h, int x, int y, float2 fa, float2 fb,
-                                             float ma[5], float mb[5]) {
-  float qa[5], qb[5];
-  {
-    const float* q = padd(R0, y * w + x);
-#pragma unroll
-    for (int c = 0; c < 5; ++c) { qa[c] = __ldg(q); qb[c] = __ldg(padd(q, w)); q = padd(q, n); }
-  }
-  float fxa = (float)x + fa.x, fya = (float)y + fa.y;
-  float fxb = (float)x + fb.x, fyb = (float)(y + 1) + fb.y;
-  const int x1a = __float2int_rd(fxa), y1a = __float2int_rd(fya);
-  const int x1b = __float2int_rd(fxb), y1b = __float2int_rd(fyb);
-  const bool ina = (unsigned)x1a < (unsigned)(w - 1) && (unsigned)y1a < (unsigned)(h - 1);
-  const bool inb = (unsigned)x1b < (unsigned)(w - 1) && (unsigned)y1b < (unsigned)(h - 1);
-  if (ina && inb && x1b == x1a && y1b == y1a + 1) {
-    fxa -= (float)x1a; fya -= (float)y1a; fxb -= (float)x1b; fyb -= (float)y1b;
-    const float a00 = (1.f - fxa) * (1.f - fya), a01 = fxa * (1.f - fya), a10 = (1.f - fxa) * fya, a11 = fxa * fya;
-    const float b00 = (1.f - fxb) * (1.f - fyb), b01 = fxb * (1.f - fyb), b10 = (1.f - fxb) * fyb, b11 = fxb * fyb;
-    float ra[5], rb[5];
-    if (fits) {
-      const float* p = win + (y1a - wy0) * kWinW + (x1a - wx0);
-#pragma unroll
-      for (int pl = 0; pl < 5; ++pl) {
-        const float t00 = p[pl * kWinPlaneFloats], t01 = p[pl * kWinPlaneFloats + 1];
-        const float t10 = p[pl * kWinPlaneFloats + kWinW], t11 = p[pl * kWinPlaneFloats + kWinW + 1];
-        const float t20 = p[pl * kWinPlaneFloats + 2 * kWinW], t21 = p[pl * kWinPlaneFloats + 2 * kWinW + 1];
-        ra[pl] = a00 * t00 + a01 * t01 + a10 * t10 + a11 * t11;
-        rb[pl] = b00 * t10 + b01 * t11 + b10 * t20 + b11 * t21;
-      }
-    } else {
-      const float* p = padd(R1, y1a * w + x1a);
-#pragma unroll
-      for (int pl = 0; pl < 5; ++pl) {
-        const float* p1 = padd(p, w);
-        const float* p2 = padd(p1, w);
-        const float t00 = __ldg(p), t01 = __ldg(p + 1);
-        const float t10 = __ldg(p1), t11 = __ldg(p1 + 1);
-        const float t20 = __ldg(p2), t21 = __ldg(p2 + 1);
-        ra[pl] = a00 * t00 + a01 * t01 + a10 * t10 + a11 * t11;
-        rb[pl] = b00 * t10 + b01 * t11 + b10 * t20 + b11 * t21;
-        p = padd(p, n);
-      }
-    }
-    um_finish(qa[0], qa[1], qa[2], qa[3], qa[4], true, ra[0], ra[1], ra[2], ra[3], ra[4], w, h, x, y, fa.x, fa.y, ma);
-    um_finish(qb[0], qb[1], qb[2], qb[3], qb[4], true, rb[0], rb[1], rb[2], rb[3], rb[4], w, h, x, y + 1, fb.x, fb.y, mb);
-  } else {
-    update_matrices_q(qa[0], qa[1], qa[2], qa[3], qa[4], R1, n, w, h, x, y, fa.x, fa.y, ma);
-    update_matrices_q(qb[0], qb[1], qb[2], qb[3], qb[4], R1, n, w, h, x, y + 1, fb.x, fb.y, mb);
-  }
-}
 
 __global__ void __launch_bounds__(kFiThreads, 4)
 iter15_win_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ Mout, const float* __restrict__ R,
@@ -1825,69 +1790,12 @@ iter15_win_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ M
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   int btx, bty, bpz;
-  int bid;
-  tile_of_block(ord, btx, bty, bpz, bid);
+  tile_of_band_order(ord, (int)blockIdx.x, btx, bty, bpz);
   const int pair = pair0 + bpz;
   const int ox0 = btx * kFiTW, oy0 = bty * kFiTH;
-  const int bx0 = ox0 - kFiM - 1, by0 = oy0 - kFiM;
 
-  if (tid == 0) {
-    tma_mbar_init(&bars[0], 1);
-    tma_mbar_init(&bars[1], 1);
-    tma_mbar_init(&bars[2], 1);
-#ifndef STB_CPU_EMU
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-#endif
-  }
-  __syncthreads();
-  if (tid == 0) {
-    tma_load_tile(raw[0], &map_in, bx0, by0, pair * 5 + 0, &bars[0]);
-    tma_load_tile(raw[1], &map_in, bx0, by0, pair * 5 + 1, &bars[1]);
-  }
-  if (prefetch_R && tid >= 32 && tid < ((ord.band == 0 || ord.band == -2 || bpz == ord.np - 1) ? 42 : 37))
-    tma_prefetch_l2(&map_R, ox0, oy0, pair * 5 + (tid - 32));
-
-  // ---- box phase: identical to iter15_tma_kernel
-  const int vg = tid >> 6, vcx = tid & 63;
-  const bool vact = vcx < kFiRawW;
-  const bool border = (bx0 + 1 < 0) || (by0 < 0) || (bx0 + 1 + kFiRawW > w) || (by0 + kTmRawH > h);
-  const int ccol = min(max(bx0 + 1 + vcx, 0), w - 1) - bx0;
   float sums[5][kFiGC];
-#pragma unroll
-  for (int c = 0; c < 5; ++c) {
-    const int st = c & 1;
-    tma_mbar_wait(&bars[st], (unsigned)((c >> 1) & 1));
-    float* vt = Vt[st];
-    if (vact) {
-      float v[kFiRows];
-      if (!border) {
-        const float* col = &raw[st][(vg * 8) * kTmRawW + vcx + 1];
-#pragma unroll
-        for (int j = 0; j < kFiRows; ++j) v[j] = col[j * kTmRawW];
-      } else {
-#pragma unroll
-        for (int j = 0; j < kFiRows; ++j) {
-          const int rr = min(max(by0 + vg * 8 + j, 0), h - 1) - by0;
-          v[j] = raw[st][rr * kTmRawW + ccol];
-        }
-      }
-      float vs[8];
-      box15<8>(v, vs);
-      float* o = vt + vcx * 33 + vg * 8;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) o[i] = vs[i];
-    }
-    __syncthreads();
-    if (tid == 0 && c + 2 < 5) tma_load_tile(raw[st], &map_in, bx0, by0, pair * 5 + c + 2, &bars[st]);
-    {
-      const float* rowp = vt + (warp * kFiGC) * 33 + lane;
-      float t[kFiGC + 14];
-#pragma unroll
-      for (int j = 0; j < kFiGC + 14; ++j) t[j] = rowp[j * 33];
-      box15<kFiGC>(t, sums[c]);
-    }
-  }
-  __syncthreads();   // every read of raw / Vt is done before fl and the window overlay them
+  iter15_tma_box<3>(raw, Vt, bars, &map_in, &map_R, prefetch_R != 0, bpz == ord.np - 1, w, h, pair, ox0, oy0, sums);
 
   // ---- solve + bounding box of the bilinear footprints of this thread's pixels (row oy0 + lane, columns ox0 + 6 warp ..)
   int minx = 0x7fffffff, miny = 0x7fffffff, maxx = -1, maxy = -1;
@@ -1895,8 +1803,7 @@ iter15_win_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ M
     const int y = oy0 + lane;
 #pragma unroll
     for (int i = 0; i < kFiGC; ++i) {
-      const float2 f = solve_flow15(sums[0][i], sums[1][i], sums[2][i], sums[3][i], sums[4][i]);
-      fl[lane * kFiFlStride + warp * kFiGC + i] = f;
+      const float2 f = stage_flow15(fl, sums, i);
       const int x = ox0 + warp * kFiGC + i;
       if (x < w && y < h) {
         const int x1 = __float2int_rd((float)x + f.x), y1 = __float2int_rd((float)y + f.y);
@@ -1937,35 +1844,10 @@ iter15_win_kernel(const STB_GRID_CONSTANT TmaMap3D map_in, float* __restrict__ M
     }
   }
 
-  // ---- update phase: vertical pixel pairs, consecutive lanes on consecutive x
-  const size_t n = (size_t)w * h;
-  const int ni = (int)n;
-  const float* R0 = R + (size_t)pair * 5 * n;
-  const float* R1 = R0 + 5 * n;
-  float* Mp = Mout + (size_t)pair * 5 * n;
+  // ---- update phase: vertical pixel pairs through the window when it fits
   tma_mbar_wait(&bars[2], 0u);
-  const int wx0 = wprm[0], wy0 = wprm[1];
-  const bool fits = wprm[2] != 0;
-#pragma unroll 1
-  for (int i = 0; i < (kFiTW * kFiTH) / (2 * kFiThreads); ++i) {
-    const int p2 = tid + i * kFiThreads;
-    const int tp = p2 / kFiTW, tx = p2 - tp * kFiTW;
-    const int x = ox0 + tx, y = oy0 + 2 * tp;
-    if (x >= w || y >= h) continue;
-    const float2 fa = fl[(2 * tp) * kFiFlStride + tx];
-    const float2 fb = fl[(2 * tp + 1) * kFiFlStride + tx];
-    float* Mo = Mp + (y * w + x);
-    float ma[5], mb[5];
-    if (y + 1 < h) {
-      um_vpair_win(R0, R1, win, wx0, wy0, fits, ni, w, h, x, y, fa, fb, ma, mb);
-#pragma unroll
-      for (int c = 0; c < 5; ++c) { *Mo = ma[c]; *padd(Mo, w) = mb[c]; Mo = padd(Mo, ni); }
-    } else {
-      update_matrices_px(R0, R1, ni, w, h, x, y, fa.x, fa.y, ma);
-#pragma unroll
-      for (int c = 0; c < 5; ++c) Mo[c * ni] = ma[c];
-    }
-  }
+  const R1Win rw = {win, wprm[0], wprm[1], wprm[2] != 0};
+  iter15_global_phase<true, false>(fl, nullptr, Mout, R, rw, PtrBatch<float>{}, nullptr, w, h, pair, bpz, ox0, oy0);
 }
 
 }  // namespace stb
@@ -1986,13 +1868,8 @@ struct stb_farneback {
   PyrParams pyr[kMaxScales];
   MergedTaps merged[kMaxScales];
   int pow2[kMaxScales];
-  int chunk[kMaxScales];
   int fast_pyr;          // levels 1.. from one horizontal + one vertical launch (pyr_h_kernel / pyr_v_kernel)
   PyrTaps3 taps3;
-  int init_prefetch_waves;   // updmat_init_kernel's prefetch distance in resident waves
-  int old_pyr0;              // A/B knob: the 4 x 4-patch pyr0_kernel instead of pyr0x8_kernel
-  int init_minb;             // experiment knob: updmat_init_kernel's minimum blocks per SM (register cap 48 / 64 / 80)
-  int band_iter, band_init;  // TileOrder.band of the iteration kernels (tile rows of 32 px) / updmat_init_kernel (rows of 8 px); 0 = round-1 order
   // device workspace
   uint8_t* gray;    // [F][H*W]
   float* I;         // [F][N_k]      (N_0 sized)
@@ -2001,7 +1878,6 @@ struct stb_farneback {
                            // produced ahead of (and concurrently with) the displacement iterations of the coarser levels
   cudaStream_t s_prep;     // second lane: gray -> pyramid -> polynomial expansions of every level (low priority)
   cudaEvent_t ev_fork, ev_R[kMaxScales];
-  int two_lanes;
   // CUDA-graph replay of a whole batch (see graph_run): one instantiated graph per (pairs, outputs) shape
   int use_graph;
   cudaStream_t s_cap;
@@ -2267,44 +2143,15 @@ int stb_farneback_create(int width, int height, int max_pairs, const stb_farneba
                   q.w == (width >> k) && q.h == (height >> k) && q.r == expect_r) ? 1 : 0;
     for (int t = 0; t <= ksize; ++t)
       h->merged[k].c[t] = 0.5f * ((t < ksize ? q.taps[t] : 0.f) + (t > 0 ? q.taps[t - 1] : 0.f));
-    // Pairs per launch: the whole batch (up to the pointer-table size).  Measured on B200 (1080p,
-    // 16-pair batches): 1 pair per level-0 launch 3585 fps, 2 -> 3944, 4 -> 4276, 8 -> 4499.  The
-    // kernels are issue/latency bound, so wave quantisation and launch tails (1360 blocks over
-    // 592 resident slots = 2.3 waves for one 1080p pair) cost more than keeping one pair's
-    // working set (~92 B/px) resident in the 126 MB L2 buys.
-    int c = kMaxPtrBatch;
-    h->chunk[k] = c;
   }
   {
     // two-launch pyramid for levels >= 1: every level an exact power-of-two size, 32-pixel segments
-    bool ok = h->nscales >= 2 && (width % 32) == 0 && !getenv("STB_NO_FAST_PYR");
+    bool ok = h->nscales >= 2 && (width % 32) == 0;
     for (int k = 1; k < h->nscales; ++k) ok = ok && h->pow2[k];
     h->fast_pyr = ok ? 1 : 0;
     for (int t = 0; t < 4; ++t) h->taps3.c1[t] = h->nscales > 1 ? h->merged[1].c[t] : 0.f;
     for (int t = 0; t < 10; ++t) h->taps3.c2[t] = h->nscales > 2 ? h->merged[2].c[t] : 0.f;
     for (int t = 0; t < 20; ++t) h->taps3.c3[t] = h->nscales > 3 ? h->merged[3].c[t] : 0.f;
-    h->init_prefetch_waves = 2;
-    // measured on B200 (1080p, 16-pair batches, one box, back to back): round-1 order through a 1-D grid 5117 fps;
-    // iteration kernels band 2 / 4 / 8 / all rows: 5284 / 5308 / 5317 / 5001; updmat_init_kernel band 8 / 16 / 32 /
-    // all rows: 5309 / 5308 / 5314 / 5193 and, as a 3-D grid (pair, tile x, tile y) in the hardware's own
-    // rasterisation order: +1.5 % on top (5466 vs 5383) -- the iteration kernels lose 0.4 % that way.
-    h->band_iter = 4;
-    h->band_init = -1;
-    h->init_minb = 5;
-    h->old_pyr0 = getenv("STB_OLD_PYR0") ? 1 : 0;
-    if (const char* env = getenv("STB_INIT_MINB")) h->init_minb = atoi(env);
-    if (const char* env = getenv("STB_BAND_ITER")) h->band_iter = atoi(env);
-    if (const char* env = getenv("STB_BAND_INIT")) h->band_init = atoi(env);
-    if (const char* env = getenv("STB_INIT_PREFETCH_WAVES")) h->init_prefetch_waves = atoi(env);
-  }
-  if (const char* env = getenv("STB_CHUNKS")) {   // experiment knob: "c0,c1,c2,c3" pairs per launch per level
-    int k = 0;
-    for (const char* pch = env; *pch && k < h->nscales; ++k) {
-      const int v = atoi(pch);
-      if (v >= 1 && v <= kMaxPtrBatch) h->chunk[k] = v;
-      while (*pch && *pch != ',') ++pch;
-      if (*pch == ',') ++pch;
-    }
   }
   const WsLayout l = ws_layout(width, height, max_pairs, h->nscales, h->w, h->h);
   uint8_t* base = nullptr;
@@ -2334,23 +2181,21 @@ int stb_farneback_create(int width, int height, int max_pairs, const stb_farneba
   h->flow[0] = (float*)(base + off); off += l.flow;
   h->flow[1] = (float*)(base + off); off += l.flow;
   {
-    const char* no_tma = getenv("STB_NO_TMA");   // A/B knob: fall back to the LDG variant
+    // STB_NO_WIN selects iter15_tma_kernel, the global-gather reference the window kernel is tested against
+    const bool no_win = getenv("STB_NO_WIN") != nullptr;
     for (int k = 0; k < h->nscales; ++k) {
-      h->use_tma[k] = 0;
-      if (no_tma && no_tma[0] == '1') continue;
       // one box (64 x 46) must make sense for the level; tiny levels keep the LDG kernel
       if (h->w[k] < kTmRawW || h->h[k] < 8) continue;
       if (make_tmap(&h->tmap[0][k], h->M[0], h->w[k], h->h[k], 5 * max_pairs) &&
           make_tmap(&h->tmap[1][k], h->M[1], h->w[k], h->h[k], 5 * max_pairs))
         h->use_tma[k] = 1;
-      if (h->use_tma[k] && !getenv("STB_NO_R_PREFETCH") && h->h[k] >= kPfBoxH &&
+      if (h->use_tma[k] && h->h[k] >= kPfBoxH &&
           make_tmap(&h->tmapR[k], h->Rk[k], h->w[k], h->h[k], 5 * (max_pairs + 1), kPfBoxW, kPfBoxH))
         h->prefetch_R[k] = 1;
-      if (h->use_tma[k] && h->prefetch_R[k] && !getenv("STB_NO_WIN") && h->w[k] >= kWinW && h->h[k] >= kWinH &&
+      if (h->use_tma[k] && h->prefetch_R[k] && !no_win && h->w[k] >= kWinW && h->h[k] >= kWinH &&
           make_tmap(&h->tmapRw[k], h->Rk[k], h->w[k], h->h[k], 5 * (max_pairs + 1), kWinW, kWinH))
         h->use_win[k] = 1;
-      if (!(no_tma && no_tma[0] == '1') && !getenv("STB_NO_INIT_PREFETCH") &&
-          make_tmap(&h->tmapRi[k], h->Rk[k], h->w[k], h->h[k], 5 * (max_pairs + 1), 64, kPfInitBoxH))
+      if (make_tmap(&h->tmapRi[k], h->Rk[k], h->w[k], h->h[k], 5 * (max_pairs + 1), 64, kPfInitBoxH))
         h->prefetch_Ri[k] = 1;
     }
   }
@@ -2375,8 +2220,7 @@ int stb_farneback_create(int width, int height, int max_pairs, const stb_farneba
   {
     // second lane for the pyramid / polynomial-expansion chain (see run_levels); lowest priority, so the
     // displacement-iteration chain is scheduled first whenever both have blocks ready
-    h->two_lanes = getenv("STB_ONE_LANE") ? 0 : 1;
-    h->use_graph = getenv("STB_NO_GRAPH") ? 0 : 1;
+    h->use_graph = getenv("STB_NO_GRAPH") ? 0 : 1;   // direct launches, the reference the graph replay is tested against
     int lo = 0, hi = 0;
     cudaError_t e2 = cudaDeviceGetStreamPriorityRange(&lo, &hi);
     if (e2 == cudaSuccess) e2 = cudaStreamCreateWithPriority(&h->s_prep, cudaStreamNonBlocking, lo);
@@ -2469,8 +2313,6 @@ static inline bool fused_hist_available(const stb_farneback* h) {
   return h->prm.win_size / 2 == kFiM && (h->prm.flags & kFlagGaussian) == 0;
 }
 
-// d_hist != NULL: fused FlowHistogram (n*128 int32, pre-zeroed) when the winSize-15 kernel runs;
-// returns through *hist_fused whether it did.  d_flow entries may be NULL only in that case.
 // I_k and R_k of frames [fa, fb) at level k on stream `sp` (the "prep" work of a level)
 static int prep_level(stb_farneback* h, int k, int fa, int fb, bool fastpyr, cudaStream_t sp) {
   const int w = h->w[k], hh = h->h[k];
@@ -2485,7 +2327,7 @@ static int prep_level(stb_farneback* h, int k, int fa, int fb, bool fastpyr, cud
     // I_k already produced by pyr_h_kernel / pyr_v_kernel
   } else if (k == 0) {
     // rows of the gray plane and of I are 4/16-byte aligned iff W % 4 == 0 (bases are 256-byte aligned)
-    if ((w % 8) == 0 && !h->old_pyr0)
+    if ((w % 8) == 0)
       stb_launch(pyr0x8_kernel, dim3(ceil_div(w, 256), ceil_div(hh, 8 * kPyr0Rows), fb - fa), dim3(256), 0, sp,
                  (const uint8_t*)h->gray, h->I, w, hh, pp.taps[0], pp.taps[1], pp.taps[2], fa);
     else
@@ -2536,10 +2378,9 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
   // Levels >= 1 of all n + 1 frames from two launches (the intermediate lives in the level-0 R buffer, which is
   // not written before the level-0 polynomial expansion; I_1.. are packed into the I buffer, which level 0
   // only overwrites after they have been consumed).  Needs the batch in one chunk at every level.
-  bool one_chunk = true;
-  for (int k = 0; k < h->nscales; ++k) one_chunk = one_chunk && n <= h->chunk[k];
+  const bool one_chunk = n <= kMaxPtrBatch;
   const bool fastpyr = h->fast_pyr != 0 && one_chunk;
-  const bool lanes = h->two_lanes != 0 && one_chunk && h->dbg_level < 0;
+  const bool lanes = one_chunk && h->dbg_level < 0;
   const size_t N0 = (size_t)h->W * h->H;
   cudaStream_t sp = s;
   if (lanes) {
@@ -2579,8 +2420,13 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
     int frames_done = 0;
     const bool dbg = (h->dbg_level == k);
     if (lanes) STB_CUDA(cudaStreamWaitEvent(s, h->ev_R[k], 0));
-    for (int p0 = 0; p0 < n; p0 += h->chunk[k]) {
-      const int p1 = (p0 + h->chunk[k] < n) ? p0 + h->chunk[k] : n;
+    // Pairs per launch: the whole batch (up to the pointer-table size).  Measured on B200 (1080p,
+    // 16-pair batches): 1 pair per level-0 launch 3585 fps, 2 -> 3944, 4 -> 4276, 8 -> 4499.  The
+    // kernels are issue/latency bound, so wave quantisation and launch tails (1360 blocks over
+    // 592 resident slots = 2.3 waves for one 1080p pair) cost more than keeping one pair's
+    // working set (~92 B/px) resident in the 126 MB L2 buys.
+    for (int p0 = 0; p0 < n; p0 += kMaxPtrBatch) {
+      const int p1 = (p0 + kMaxPtrBatch < n) ? p0 + kMaxPtrBatch : n;
       const int np = p1 - p0;
       // frames [fa, fb) still need I_k and R_k
       const int fa = frames_done, fb = p1 + 1;
@@ -2589,16 +2435,12 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
         if (prc) return prc;
         frames_done = fb;
       }
-      (void)F;
       {
-        // prefetch distance: about two resident waves expressed in block rows
-        const int bx = ceil_div(w, 64), by = ceil_div(hh, 8);
-        // prefetch distance: about `init_prefetch_waves` resident waves (5 blocks per SM) in blocks of the 1-D grid
-        const int ahead = h->prefetch_Ri[k] ? h->init_prefetch_waves * 4 * num_sms() : 0;
-        const TileOrder oi = {bx, by, np, h->band_init};
-        auto* init_fn = h->init_minb == 4 ? updmat_init_kernel<4> : (h->init_minb == 3 ? updmat_init_kernel<3> : updmat_init_kernel<5>);
-        stb_launch(init_fn, oi.band == -2 ? dim3(bx, by, np) : oi.band < 0 ? dim3(np, bx, by) : dim3((unsigned)(bx * by * np)), dim3(256), 0, s, Rk,
-                   coarse, h->M[0], w, hh, wc, hc, up_sx, up_sy, (float)(1. / h->prm.pyr_scale), p0, h->tmapRi[k], ahead, oi);
+        // prefetch distance in blocks of the grid's linear order: two resident waves of 4 blocks per SM
+        // (the occupancy it was tuned at; about 1.6 waves at the kernel's 5)
+        const int ahead = h->prefetch_Ri[k] ? 2 * 4 * num_sms() : 0;
+        stb_launch(updmat_init_kernel, dim3(np, ceil_div(w, 64), ceil_div(hh, 8)), dim3(256), 0, s, Rk, coarse, h->M[0], w, hh,
+                   wc, hc, up_sx, up_sy, (float)(1. / h->prm.pyr_scale), p0, h->tmapRi[k], ahead);
       }
       STB_CHECK_LAUNCH("updmat_init_kernel");
       if (dbg && h->dbg_pair >= p0 && h->dbg_pair < p1) {
@@ -2616,10 +2458,8 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
       int mc = 0;
       const bool gauss = (h->prm.flags & kFlagGaussian) != 0;
       const bool fast15 = (m == kFiM) && !gauss;   // the winSize-15 kernels are box-window only
-      const TileOrder ot = {ceil_div(w, kFiTW), ceil_div(hh, kFiTH), np, h->band_iter};
-      const dim3 grid = fast15 ? (ot.band == -2 ? dim3(ot.tiles_x, ot.tiles_y, np)
-                                                : ot.band < 0 ? dim3(np, ot.tiles_x, ot.tiles_y) : dim3((unsigned)(ot.tiles_x * ot.tiles_y * np)))
-                               : dim3(ceil_div(w, kItTW), ceil_div(hh, kItTH), np);
+      const TileOrder ot = {ceil_div(w, kFiTW), ceil_div(hh, kFiTH), np};
+      const dim3 grid = fast15 ? dim3((unsigned)(ot.tiles_x * ot.tiles_y * np)) : dim3(ceil_div(w, kItTW), ceil_div(hh, kItTH), np);
       const bool prof = h->profile && k == 0 && h->prm.num_iters > 1;
       for (int it = 0; it < h->prm.num_iters; ++it) {
         if (it < h->prm.num_iters - 1) {
@@ -2756,9 +2596,7 @@ static void graph_free(FbGraph* g) {
 static bool graph_eligible(const stb_farneback* h, int n) {
   if (!h->use_graph || h->profile || h->dbg_level >= 0 || !h->s_cap) return false;
   if (!fused_hist_available(h) || !h->use_tma[0]) return false;
-  for (int k = 0; k < h->nscales; ++k)
-    if (n > h->chunk[k]) return false;
-  return n + 1 <= kMaxPtrBatch;      // one gray launch
+  return n + 1 <= kMaxPtrBatch;      // one gray launch (and so one chunk per level)
 }
 
 // enqueue of one batch on `s` (shared by the direct path and the capture)

@@ -396,7 +396,6 @@ static int launch_hist(Addr addr, int n, unsigned long long nbytes, int32_t* d_o
   // slots, one block per frame.
   const long long max_useful = (long long)((nvec + (unsigned long long)kHistThreads * 4 - 1) / ((unsigned long long)kHistThreads * 4));
   long long total = wave;
-  if (const char* env = getenv("STB_HIST_WAVES")) { const int k = atoi(env); if (k >= 1 && k <= 16) total = (long long)wave * k; }
   if (total < n) total = n;
   if (max_useful >= 1 && total > max_useful * n) total = max_useful * n;
   if (total < n) total = n;
