@@ -1872,7 +1872,8 @@ struct stb_farneback {
   PyrTaps3 taps3;
   // device workspace
   uint8_t* gray;    // [F][H*W]
-  float* I;         // [F][N_k]      (N_0 sized)
+  float* I;         // [F][N_0] slots: I_k of frame f at I + I_off[k] + f * I_stride[k]
+  size_t I_off[kMaxScales], I_stride[kMaxScales];
   float* R;         // [F][5][N_0]   level 0 (and, before its expansion is written, the pyramid's intermediate)
   float* Rk[kMaxScales];   // [F][5][N_k] per level: Rk[0] = R; separate buffers so that the expansions of all levels can be
                            // produced ahead of (and concurrently with) the displacement iterations of the coarser levels
@@ -2152,6 +2153,15 @@ int stb_farneback_create(int width, int height, int max_pairs, const stb_farneba
     for (int t = 0; t < 4; ++t) h->taps3.c1[t] = h->nscales > 1 ? h->merged[1].c[t] : 0.f;
     for (int t = 0; t < 10; ++t) h->taps3.c2[t] = h->nscales > 2 ? h->merged[2].c[t] : 0.f;
     for (int t = 0; t < 20; ++t) h->taps3.c3[t] = h->nscales > 3 ? h->merged[3].c[t] : 0.f;
+    // pyr_v_kernel packs I_1, I_2, .. one after the other into the frame's N_0 slot; the per-level
+    // kernels give every level its own dense [F][N_k] layout
+    size_t packed = 0;
+    for (int k = 0; k < h->nscales; ++k) {
+      const bool in_slot = h->fast_pyr && k >= 1;
+      h->I_off[k] = in_slot ? packed : 0;
+      h->I_stride[k] = in_slot ? (size_t)width * height : (size_t)h->w[k] * h->h[k];
+      if (in_slot) packed += (size_t)h->w[k] * h->h[k];
+    }
   }
   const WsLayout l = ws_layout(width, height, max_pairs, h->nscales, h->w, h->h);
   uint8_t* base = nullptr;
@@ -2314,16 +2324,12 @@ static inline bool fused_hist_available(const stb_farneback* h) {
 }
 
 // I_k and R_k of frames [fa, fb) at level k on stream `sp` (the "prep" work of a level)
-static int prep_level(stb_farneback* h, int k, int fa, int fb, bool fastpyr, cudaStream_t sp) {
+static int prep_level(stb_farneback* h, int k, int fa, int fb, cudaStream_t sp) {
   const int w = h->w[k], hh = h->h[k];
-  const size_t nk = (size_t)w * hh;
-  const size_t N0 = (size_t)h->W * h->H;
   const PyrParams& pp = h->pyr[k];
-  size_t i_off = 0;
-  if (fastpyr) for (int j = 1; j < k; ++j) i_off += (size_t)h->w[j] * h->h[j];
-  const float* Ik = h->I + i_off;
-  const size_t i_stride = (fastpyr && k >= 1) ? N0 : nk;
-  if (fastpyr && k >= 1) {
+  const float* Ik = h->I + h->I_off[k];
+  const size_t i_stride = h->I_stride[k];
+  if (h->fast_pyr && k >= 1) {
     // I_k already produced by pyr_h_kernel / pyr_v_kernel
   } else if (k == 0) {
     // rows of the gray plane and of I are 4/16-byte aligned iff W % 4 == 0 (bases are 256-byte aligned)
@@ -2356,70 +2362,72 @@ static int prep_level(stb_farneback* h, int k, int fa, int fb, bool fastpyr, cud
   return STB_OK;
 }
 
-// d_hist != NULL: fused FlowHistogram (n*128 int32, pre-zeroed) when the winSize-15 kernel runs;
-// returns through *hist_fused whether it did.  d_flow entries may be NULL only in that case.
+// d_hist != NULL: fused FlowHistogram (n*128 int32, pre-zeroed) in the level-0 last iteration, for parameter
+// sets with fused_hist_available(h) only; then d_flow entries may be NULL.
 //
 // Schedule.  A level needs (a) I_k and the polynomial expansion R_k of every frame -- which depend on the
 // gray planes only -- and (b) the chain updmat_init -> iterations, which depends on R_k and on the coarser
-// level's flow.  When the whole batch fits one launch per level, (a) for ALL levels runs on the handle's own
-// low-priority stream (forked from the caller's stream after the gray conversion, every R_k in its own
-// buffer) while the caller's stream walks the chain (b) from the coarsest level, waiting per level on an
-// event: the small, latency-bound launches of the coarse levels (less than one resident wave at level 3)
-// share the GPU with the bandwidth-heavy expansion of the fine levels instead of running alone.  The lanes
-// join before the call returns control of the stream.  Batches that need several chunks per level (more
-// than 64 pairs per call) and the debug taps use the single-lane order.
-static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_t s, int32_t* d_hist = nullptr,
-                      bool* hist_fused = nullptr) {
-  if (hist_fused) *hist_fused = (d_hist != nullptr) && fused_hist_available(h);
+// level's flow.  (a) for ALL levels runs on the handle's own low-priority stream (forked from the caller's
+// stream after the gray conversion, every R_k in its own buffer) while the caller's stream walks the chain
+// (b) from the coarsest level in pointer-table chunks of pairs, waiting per level on an event: the small,
+// latency-bound launches of the coarse levels (less than one resident wave at level 3) share the GPU with
+// the bandwidth-heavy expansion of the fine levels instead of running alone.  The caller's stream waits on
+// the level-0 event, recorded last, so the lanes join before the call returns control of the stream.
+// The debug taps of I_k / R_k are copied on the prep lane right after level k's prep: with the two-launch
+// pyramid I_k (k >= 1) lives in the frame's level-0 slot, which the level-0 pyramid overwrites next.
+static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_t s, int32_t* d_hist = nullptr) {
   const int F = n + 1;
+  const int slice = kMaxPtrBatch + 1;    // frames per prep launch: a batch of up to 64 pairs is one slice
   const int m = h->prm.win_size / 2;
   const size_t it_smem = iter_smem_bytes(m);
   int fl_cur = 0;  // h->flow[fl_cur] receives this level's flow (levels >= 1)
-  // Levels >= 1 of all n + 1 frames from two launches (the intermediate lives in the level-0 R buffer, which is
-  // not written before the level-0 polynomial expansion; I_1.. are packed into the I buffer, which level 0
-  // only overwrites after they have been consumed).  Needs the batch in one chunk at every level.
-  const bool one_chunk = n <= kMaxPtrBatch;
-  const bool fastpyr = h->fast_pyr != 0 && one_chunk;
-  const bool lanes = one_chunk && h->dbg_level < 0;
-  const size_t N0 = (size_t)h->W * h->H;
-  cudaStream_t sp = s;
-  if (lanes) {
-    sp = h->s_prep;
-    STB_CUDA(cudaEventRecord(h->ev_fork, s));            // gray planes ready; the previous call on `s` is done with R / I
-    STB_CUDA(cudaStreamWaitEvent(sp, h->ev_fork, 0));
-  }
-  if (fastpyr) {
+  const bool dbg_in_batch = h->dbg_pair >= 0 && h->dbg_pair < n;
+  cudaStream_t sp = h->s_prep;
+  STB_CUDA(cudaEventRecord(h->ev_fork, s));            // gray planes ready; the previous call on `s` is done with R / I
+  STB_CUDA(cudaStreamWaitEvent(sp, h->ev_fork, 0));
+  if (h->fast_pyr) {
+    // Levels >= 1 from two launches per slice.  The intermediate lives in the level-0 R buffer, which is not
+    // written before the level-0 polynomial expansion; I_1.. are packed into the I slots, which the level-0
+    // pyramid only overwrites after every level >= 1 has been expanded.
     const int nlev = h->nscales - 1;
     const int items = (h->W >> 5) * h->H;
-    stb_launch(pyr_h_kernel, dim3(ceil_div(items, 128), F), dim3(128), 0, sp, (const uint8_t*)h->gray, h->R, h->W, h->H, h->taps3, nlev, 0);
-    STB_CHECK_LAUNCH("pyr_h_kernel");
     int quads = 0;
     for (int k = 1; k <= nlev; ++k) quads += (h->w[k] >> 2) * h->h[k];
-    stb_launch(pyr_v_kernel, dim3(ceil_div(quads, 128), F), dim3(128), 0, sp, (const float*)h->R, h->I, h->W, h->H, h->taps3, nlev, N0, 0);
-    STB_CHECK_LAUNCH("pyr_v_kernel");
-  }
-  if (lanes) {
-    for (int k = h->nscales - 1; k >= 0; --k) {
-      int prc = prep_level(h, k, 0, F, fastpyr, sp);
-      if (prc) return prc;
-      STB_CUDA(cudaEventRecord(h->ev_R[k], sp));
+    for (int f0 = 0; f0 < F; f0 += slice) {
+      const int nf = (f0 + slice < F ? f0 + slice : F) - f0;
+      stb_launch(pyr_h_kernel, dim3(ceil_div(items, 128), nf), dim3(128), 0, sp, (const uint8_t*)h->gray, h->R, h->W, h->H, h->taps3,
+                 nlev, f0);
+      STB_CHECK_LAUNCH("pyr_h_kernel");
+      stb_launch(pyr_v_kernel, dim3(ceil_div(quads, 128), nf), dim3(128), 0, sp, (const float*)h->R, h->I, h->W, h->H, h->taps3, nlev,
+                 h->I_stride[1], f0);
+      STB_CHECK_LAUNCH("pyr_v_kernel");
     }
+  }
+  for (int k = h->nscales - 1; k >= 0; --k) {
+    for (int f0 = 0; f0 < F; f0 += slice) {
+      int prc = prep_level(h, k, f0, f0 + slice < F ? f0 + slice : F, sp);
+      if (prc) return prc;
+    }
+    if (h->dbg_level == k && dbg_in_batch) {
+      const size_t nk = (size_t)h->w[k] * h->h[k];
+      const float* I0 = h->I + h->I_off[k] + (size_t)h->dbg_pair * h->I_stride[k];
+      const float* R0 = h->Rk[k] + (size_t)h->dbg_pair * 5 * nk;
+      if (h->dbg_I0) STB_CUDA(cudaMemcpyAsync(h->dbg_I0, I0, nk * 4, cudaMemcpyDeviceToDevice, sp));
+      if (h->dbg_I1) STB_CUDA(cudaMemcpyAsync(h->dbg_I1, I0 + h->I_stride[k], nk * 4, cudaMemcpyDeviceToDevice, sp));
+      if (h->dbg_R0) STB_CUDA(cudaMemcpyAsync(h->dbg_R0, R0, nk * 20, cudaMemcpyDeviceToDevice, sp));
+      if (h->dbg_R1) STB_CUDA(cudaMemcpyAsync(h->dbg_R1, R0 + 5 * nk, nk * 20, cudaMemcpyDeviceToDevice, sp));
+    }
+    STB_CUDA(cudaEventRecord(h->ev_R[k], sp));
   }
   for (int k = h->nscales - 1; k >= 0; --k) {
     const int w = h->w[k], hh = h->h[k];
     const size_t nk = (size_t)w * hh;
-    // I_k of frame f: Ik + f * i_stride
-    size_t i_off = 0;
-    if (fastpyr) for (int j = 1; j < k; ++j) i_off += (size_t)h->w[j] * h->h[j];
-    const float* Ik = h->I + i_off;
-    const size_t i_stride = (fastpyr && k >= 1) ? N0 : nk;
     const float* Rk = h->Rk[k];
     const float* coarse = (k == h->nscales - 1) ? nullptr : h->flow[fl_cur ^ 1];
     const int wc = coarse ? h->w[k + 1] : 0, hc = coarse ? h->h[k + 1] : 0;
     const double up_sx = coarse ? 1. / ((double)w / wc) : 0, up_sy = coarse ? 1. / ((double)hh / hc) : 0;
-    int frames_done = 0;
     const bool dbg = (h->dbg_level == k);
-    if (lanes) STB_CUDA(cudaStreamWaitEvent(s, h->ev_R[k], 0));
+    STB_CUDA(cudaStreamWaitEvent(s, h->ev_R[k], 0));
     // Pairs per launch: the whole batch (up to the pointer-table size).  Measured on B200 (1080p,
     // 16-pair batches): 1 pair per level-0 launch 3585 fps, 2 -> 3944, 4 -> 4276, 8 -> 4499.  The
     // kernels are issue/latency bound, so wave quantisation and launch tails (1360 blocks over
@@ -2428,13 +2436,6 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
     for (int p0 = 0; p0 < n; p0 += kMaxPtrBatch) {
       const int p1 = (p0 + kMaxPtrBatch < n) ? p0 + kMaxPtrBatch : n;
       const int np = p1 - p0;
-      // frames [fa, fb) still need I_k and R_k
-      const int fa = frames_done, fb = p1 + 1;
-      if (fb > fa && !lanes) {
-        int prc = prep_level(h, k, fa, fb, fastpyr, s);
-        if (prc) return prc;
-        frames_done = fb;
-      }
       {
         // prefetch distance in blocks of the grid's linear order: two resident waves of 4 blocks per SM
         // (the occupancy it was tuned at; about 1.6 waves at the kernel's 5)
@@ -2443,14 +2444,8 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
                    wc, hc, up_sx, up_sy, (float)(1. / h->prm.pyr_scale), p0, h->tmapRi[k], ahead);
       }
       STB_CHECK_LAUNCH("updmat_init_kernel");
-      if (dbg && h->dbg_pair >= p0 && h->dbg_pair < p1) {
-        const int dp = h->dbg_pair;
-        if (h->dbg_I0) STB_CUDA(cudaMemcpyAsync(h->dbg_I0, Ik + (size_t)dp * i_stride, nk * 4, cudaMemcpyDeviceToDevice, s));
-        if (h->dbg_I1) STB_CUDA(cudaMemcpyAsync(h->dbg_I1, Ik + (size_t)(dp + 1) * i_stride, nk * 4, cudaMemcpyDeviceToDevice, s));
-        if (h->dbg_R0) STB_CUDA(cudaMemcpyAsync(h->dbg_R0, Rk + (size_t)dp * 5 * nk, nk * 20, cudaMemcpyDeviceToDevice, s));
-        if (h->dbg_R1) STB_CUDA(cudaMemcpyAsync(h->dbg_R1, Rk + (size_t)(dp + 1) * 5 * nk, nk * 20, cudaMemcpyDeviceToDevice, s));
-        if (h->dbg_M0) STB_CUDA(cudaMemcpyAsync(h->dbg_M0, h->M[0] + (size_t)dp * 5 * nk, nk * 20, cudaMemcpyDeviceToDevice, s));
-      }
+      if (dbg && h->dbg_M0 && h->dbg_pair >= p0 && h->dbg_pair < p1)
+        STB_CUDA(cudaMemcpyAsync(h->dbg_M0, h->M[0] + (size_t)h->dbg_pair * 5 * nk, nk * 20, cudaMemcpyDeviceToDevice, s));
       PtrBatch<float> fo;
       for (int i = 0; i < kMaxPtrBatch; ++i) fo.p[i] = nullptr;
       for (int i = 0; i < np; ++i)
@@ -2516,9 +2511,17 @@ static int run_levels(stb_farneback* h, int n, float* const* d_flow, cudaStream_
   return STB_OK;
 }
 
-static int check_run_args(stb_farneback* h, const void* frames, int n, const char* who) {
+// Checks the caller's tables before anything is enqueued: frames[0..n] and (when given, or always with
+// `need_flow`) d_flow[0..n-1] must not hold NULL.  An empty batch is accepted without looking at them.
+static int check_run_args(stb_farneback* h, const uint8_t* const* frames, int n, float* const* d_flow, bool need_flow, const char* who) {
   if (!h || !frames || n < 0) { set_error("%s: invalid argument", who); return STB_ERR_INVALID; }
   if (n > h->max_pairs) { set_error("%s: n=%d exceeds max_pairs=%d", who, n, h->max_pairs); return STB_ERR_INVALID; }
+  if (n == 0) return STB_OK;
+  if (need_flow && !d_flow) { set_error("%s: d_flow is NULL", who); return STB_ERR_INVALID; }
+  for (int i = 0; i <= n; ++i)
+    if (!frames[i]) { set_error("%s: frame %d is NULL", who, i); return STB_ERR_INVALID; }
+  for (int i = 0; d_flow && i < n; ++i)
+    if (!d_flow[i]) { set_error("%s: d_flow[%d] is NULL", who, i); return STB_ERR_INVALID; }
   return STB_OK;
 }
 
@@ -2543,14 +2546,22 @@ static int to_gray(stb_farneback* h, const uint8_t* const* d_rgb, int F, cudaStr
     const int mcount = F - base < kMaxPtrBatch ? F - base : kMaxPtrBatch;
     PtrBatch<const uint8_t> t;
     for (int i = 0; i < kMaxPtrBatch; ++i) t.p[i] = nullptr;
-    for (int i = 0; i < mcount; ++i) {
-      if (!d_rgb[base + i]) { set_error("stb_farneback_run: frame %d is NULL", base + i); return STB_ERR_INVALID; }
-      t.p[i] = d_rgb[base + i];
-    }
+    for (int i = 0; i < mcount; ++i) t.p[i] = d_rgb[base + i];
     stb_launch(gray_kernel, dim3((unsigned)blocks, (unsigned)mcount), dim3(256), 0, s, t, h->gray + (size_t)base * npx, npx);
     STB_CHECK_LAUNCH("gray_kernel");
   }
   return STB_OK;
+}
+
+// enqueue of one batch on `s` (shared by the direct path and the capture)
+static int enqueue_batch(stb_farneback* h, const uint8_t* const* d_rgb, int n, float* const* fl, int32_t* d_hist, cudaStream_t s) {
+  int rc = to_gray(h, d_rgb, n + 1, s);
+  if (rc) return rc;
+  if (d_hist) {
+    cudaError_t e = cudaMemsetAsync(d_hist, 0, (size_t)n * STB_FLOWHIST_INTS * sizeof(int32_t), s);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(flow_hist)");
+  }
+  return run_levels(h, n, fl, s, d_hist);
 }
 
 
@@ -2597,17 +2608,6 @@ static bool graph_eligible(const stb_farneback* h, int n) {
   if (!h->use_graph || h->profile || h->dbg_level >= 0 || !h->s_cap) return false;
   if (!fused_hist_available(h) || !h->use_tma[0]) return false;
   return n + 1 <= kMaxPtrBatch;      // one gray launch (and so one chunk per level)
-}
-
-// enqueue of one batch on `s` (shared by the direct path and the capture)
-static int enqueue_batch(stb_farneback* h, const uint8_t* const* d_rgb, int n, float* const* fl, int32_t* d_hist, cudaStream_t s) {
-  int rc = to_gray(h, d_rgb, n + 1, s);
-  if (rc) return rc;
-  if (d_hist) {
-    cudaError_t e = cudaMemsetAsync(d_hist, 0, (size_t)n * STB_FLOWHIST_INTS * sizeof(int32_t), s);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(flow_hist)");
-  }
-  return run_levels(h, n, fl, s, d_hist, nullptr);
 }
 
 static int graph_build(stb_farneback* h, const uint8_t* const* d_rgb, int n, float* const* fl, int32_t* d_hist, int kind, FbGraph** out) {
@@ -2691,8 +2691,6 @@ static int graph_run(stb_farneback* h, const uint8_t* const* d_rgb, int n, float
   for (FbGraph* c : h->graphs)
     if (c->n == n && c->kind == kind) { g = c; break; }
   if (!g) {
-    for (int i = 0; i <= n; ++i)
-      if (!d_rgb[i]) { set_error("stb_farneback_run: frame %d is NULL", i); return STB_ERR_INVALID; }
     int rc = graph_build(h, d_rgb, n, fl, d_hist, kind, &g);
     if (rc) return rc;
     if (!g) { h->use_graph = 0; return STB_OK; }       // capture not possible here: stay on direct launches
@@ -2701,11 +2699,7 @@ static int graph_run(stb_farneback* h, const uint8_t* const* d_rgb, int n, float
   }
   {
     GrayArgs& a = g->gray_args[0];
-    for (int i = 0; i < kMaxPtrBatch; ++i) a.frames.p[i] = nullptr;
-    for (int i = 0; i <= n; ++i) {
-      if (!d_rgb[i]) { set_error("stb_farneback_run: frame %d is NULL", i); return STB_ERR_INVALID; }
-      a.frames.p[i] = d_rgb[i];
-    }
+    for (int i = 0; i < kMaxPtrBatch; ++i) a.frames.p[i] = i <= n ? d_rgb[i] : nullptr;
     void* args[3] = {&a.frames, &a.gray, &a.npx};
     cudaKernelNodeParams kp = g->gray_np[0];
     kp.kernelParams = args; kp.extra = nullptr;
@@ -2741,40 +2735,29 @@ static int graph_run(stb_farneback*, const uint8_t* const*, int, float* const*, 
 extern "C" {
 
 int stb_farneback_run(stb_farneback* h, const uint8_t* const* d_rgb, int n, float* const* d_flow, stb_stream_t stream) {
-  int rc = check_run_args(h, d_rgb, n, "stb_farneback_run");
-  if (rc) return rc;
-  if (n == 0) return STB_OK;
-  if (!d_flow) { set_error("stb_farneback_run: d_flow is NULL"); return STB_ERR_INVALID; }
-  for (int i = 0; i < n; ++i)
-    if (!d_flow[i]) { set_error("stb_farneback_run: d_flow[%d] is NULL", i); return STB_ERR_INVALID; }
+  int rc = check_run_args(h, d_rgb, n, d_flow, true, "stb_farneback_run");
+  if (rc || n == 0) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   bool via_graph = false;
   rc = graph_run(h, d_rgb, n, d_flow, nullptr, 0, s, &via_graph);
   if (rc || via_graph) return rc;
-  rc = to_gray(h, d_rgb, n + 1, s);
-  if (rc) return rc;
-  return run_levels(h, n, d_flow, s);
+  return enqueue_batch(h, d_rgb, n, d_flow, nullptr, s);
 }
 
 int stb_farneback_run_gray(stb_farneback* h, const uint8_t* const* d_gray, int n, float* const* d_flow, stb_stream_t stream) {
-  int rc = check_run_args(h, d_gray, n, "stb_farneback_run_gray");
-  if (rc) return rc;
-  if (n == 0) return STB_OK;
-  if (!d_flow) { set_error("stb_farneback_run_gray: d_flow is NULL"); return STB_ERR_INVALID; }
+  int rc = check_run_args(h, d_gray, n, d_flow, true, "stb_farneback_run_gray");
+  if (rc || n == 0) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   const size_t npx = (size_t)h->W * h->H;
-  for (int i = 0; i <= n; ++i) {
-    if (!d_gray[i] || (i < n && !d_flow[i])) { set_error("stb_farneback_run_gray: NULL pointer at %d", i); return STB_ERR_INVALID; }
+  for (int i = 0; i <= n; ++i)
     STB_CUDA(cudaMemcpyAsync(h->gray + (size_t)i * npx, d_gray[i], npx, cudaMemcpyDeviceToDevice, s));
-  }
   return run_levels(h, n, d_flow, s);
 }
 
 int stb_farneback_run_hist(stb_farneback* h, const uint8_t* const* d_rgb, int n, float* const* d_flow,
                            int32_t* d_flow_hist, stb_stream_t stream) {
-  int rc = check_run_args(h, d_rgb, n, "stb_farneback_run_hist");
-  if (rc) return rc;
-  if (n == 0) return STB_OK;
+  int rc = check_run_args(h, d_rgb, n, d_flow, false, "stb_farneback_run_hist");
+  if (rc || n == 0) return rc;
   if (!d_flow_hist) { set_error("stb_farneback_run_hist: d_flow_hist is NULL"); return STB_ERR_INVALID; }
   cudaStream_t s = (cudaStream_t)stream;
   const bool fused = fused_hist_available(h);   // the winSize-15 box kernel bins the flow it produces
@@ -2783,10 +2766,7 @@ int stb_farneback_run_hist(stb_farneback* h, const uint8_t* const* d_rgb, int n,
   float** heap = nullptr;
   if (!fl) { heap = new (std::nothrow) float*[n]; if (!heap) { set_error("out of host memory"); return STB_ERR_ALLOC; } fl = heap; }
   if (d_flow) {
-    for (int i = 0; i < n; ++i) {
-      if (!d_flow[i]) { delete[] heap; set_error("stb_farneback_run_hist: d_flow[%d] is NULL", i); return STB_ERR_INVALID; }
-      fl[i] = d_flow[i];
-    }
+    for (int i = 0; i < n; ++i) fl[i] = d_flow[i];
   } else if (fused) {
     for (int i = 0; i < n; ++i) fl[i] = nullptr;       // histogram only: the flow frames never touch HBM
   } else {
@@ -2799,14 +2779,8 @@ int stb_farneback_run_hist(stb_farneback* h, const uint8_t* const* d_rgb, int n,
     rc = graph_run(h, d_rgb, n, fl, d_flow_hist, d_flow ? 1 : 2, s, &via_graph);
     if (rc || via_graph) { delete[] heap; return rc; }
   }
-  rc = to_gray(h, d_rgb, n + 1, s);
-  if (!rc && fused) {
-    cudaError_t e = cudaMemsetAsync(d_flow_hist, 0, (size_t)n * STB_FLOWHIST_INTS * sizeof(int32_t), s);
-    if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemsetAsync(flow_hist)");
-  }
-  bool did_fuse = false;
-  if (!rc) rc = run_levels(h, n, fl, s, fused ? d_flow_hist : nullptr, &did_fuse);
-  if (!rc && !did_fuse) rc = flow_hist_device(fl, n, (unsigned long long)h->W * h->H, d_flow_hist, s, true);
+  rc = enqueue_batch(h, d_rgb, n, fl, fused ? d_flow_hist : nullptr, s);
+  if (!rc && !fused) rc = flow_hist_device(fl, n, (unsigned long long)h->W * h->H, d_flow_hist, s, true);
   delete[] heap;
   return rc;
 }

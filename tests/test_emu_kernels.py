@@ -69,8 +69,11 @@ def test_emu_frame_difference(emu):
     assert np.array_equal(o, restate.frame_difference(a[0], a[1]))
 
 
-@pytest.mark.parametrize('h,w,pairs', [(120, 160, 1), (135, 240, 2), (67, 45, 1)])
+@pytest.mark.parametrize('h,w,pairs', [(120, 160, 1), (135, 240, 2), (67, 45, 1), (64, 128, 66)])
 def test_emu_farneback_vs_oracle(emu, h, w, pairs):
+    """66 pairs: two pointer-table chunks per level and two slices of pyramid / expansion launches (the
+    two-launch pyramid at 128x64).  Every pair must equal its single-pair run bit for bit, flow and fused
+    histogram."""
     clip = synth.textured_clip(3, pairs + 1, h, w)
     hd = C.c_void_p()
     assert emu.stb_farneback_create(w, h, pairs, None, C.byref(hd)) == 0
@@ -81,6 +84,15 @@ def test_emu_farneback_vs_oracle(emu, h, w, pairs):
     rc = emu.stb_farneback_run(hd, _lib.ptr_table([f.ctypes.data for f in clip]), pairs,
                                _lib.ptr_table([f.ctypes.data for f in flows]), None)
     assert rc == 0, emu.stb_last_error()
+    fh = np.zeros((pairs, 128), np.int32)
+    assert emu.stb_farneback_run_hist(hd, _lib.ptr_table([f.ctypes.data for f in clip]), pairs, None, P(fh), None) == 0
+    emu.stb_farneback_destroy(hd)
+    assert emu.stb_farneback_create(w, h, 1, None, C.byref(hd)) == 0
+    for i in range(pairs):
+        f1, fh1 = np.zeros((h, w, 2), np.float32), np.zeros(128, np.int32)
+        assert emu.stb_farneback_run_hist(hd, _lib.ptr_table([clip[i].ctypes.data, clip[i + 1].ctypes.data]), 1,
+                                          _lib.ptr_table([f1.ctypes.data]), P(fh1), None) == 0
+        assert np.array_equal(flows[i], f1) and np.array_equal(fh[i], fh1), i
     emu.stb_farneback_destroy(hd)
     for i in range(pairs):
         e = epe(flows[i], restate.optical_flow(clip[i], clip[i + 1]))

@@ -384,20 +384,23 @@ def test_farneback_goldens(torch, ops, golden):
 
 
 def test_farneback_stage_by_stage(torch, ops):
-    """I_k, R_k, M and per-level flow against the C restatement's dumps at every scale."""
-    h, w = 260, 344
-    clip = synth.textured_clip(3, 2, h, w)
-    of = ops.OpticalFlow(w, h, max_batch=1)
-    for k in range(len(of.levels())):
-        _, d = of.debug_level(dev(torch, clip), k)
-        _, r = restate.farneback(restate.gray(clip[0]), restate.gray(clip[1]), dump_level=k)
-        assert np.abs(d['I0'].cpu().numpy() - r['I0']).max() < 1e-3
-        for nm in ('R0', 'R1', 'M0'):
-            got = d[nm].cpu().numpy()
-            ref = r[nm].transpose(2, 0, 1)
-            assert np.abs(got - ref).max() <= 2e-5 * max(1.0, np.abs(ref).max()), (k, nm)
-        check_flow(d['flow'].cpu().numpy(), r['flow'], 'level %d' % k)
-    of.close()
+    """I_k, R_k, M and per-level flow against the C restatement's dumps at every scale.  344x260 builds
+    levels 1.. with the per-level pyramid kernels; 320x256 with pyr_h / pyr_v, whose I_k share the frame's
+    I slot with level 0: the debug copy must be taken before the level-0 pyramid overwrites it."""
+    for h, w in ((260, 344), (256, 320)):
+        clip = synth.textured_clip(3, 2, h, w)
+        of = ops.OpticalFlow(w, h, max_batch=1)
+        for k in range(len(of.levels())):
+            _, d = of.debug_level(dev(torch, clip), k)
+            _, r = restate.farneback(restate.gray(clip[0]), restate.gray(clip[1]), dump_level=k)
+            assert np.abs(d['I0'].cpu().numpy() - r['I0']).max() < 1e-3, (w, h, k)
+            assert np.abs(d['I1'].cpu().numpy() - r['I1']).max() < 1e-3, (w, h, k)
+            for nm in ('R0', 'R1', 'M0'):
+                got = d[nm].cpu().numpy()
+                ref = r[nm].transpose(2, 0, 1)
+                assert np.abs(got - ref).max() <= 2e-5 * max(1.0, np.abs(ref).max()), (w, h, k, nm)
+            check_flow(d['flow'].cpu().numpy(), r['flow'], 'level %d of %dx%d' % (k, w, h))
+        of.close()
 
 
 @pytest.mark.parametrize('h,w,seed', [(480, 640, 1), (240, 426, 7), (720, 1280, 2), (1080, 1920, 3), (2160, 3840, 4), (270, 478, 5)])
@@ -582,6 +585,17 @@ def test_c_abi_error_behaviour_on_device(torch, ops):
     bad = _lib.ptr_table([fr[0].data_ptr(), 0, fr[2].data_ptr()])
     assert lib.stb_farneback_run(of._h, bad, 2, ot, None) == -1 and b'NULL' in lib.stb_last_error()
     assert lib.stb_farneback_run(of._h, ft, 0, ot, None) == 0    # empty batch is a no-op
+    # a NULL past the first pointer-table chunk is rejected before anything is launched
+    big = ops.OpticalFlow(160, 120, max_batch=66)
+    big_out = torch.empty((66, 120, 160, 2), dtype=torch.float32, device='cuda')
+    bad = _lib.ptr_table([fr[i % 4].data_ptr() if i != 65 else 0 for i in range(67)])
+    bot = _lib.ptr_table([big_out[i].data_ptr() for i in range(66)])
+    hist = torch.empty((66, 2, 64), dtype=torch.int32, device='cuda')
+    l0 = lib.stb_launch_count()
+    assert lib.stb_farneback_run(big._h, bad, 66, bot, None) == -1 and b'NULL' in lib.stb_last_error()
+    assert lib.stb_farneback_run_hist(big._h, bad, 66, bot, C.c_void_p(hist.data_ptr()), None) == -1 and b'NULL' in lib.stb_last_error()
+    assert lib.stb_launch_count() == l0
+    big.close()
     assert lib.stb_hist_rgb16_strided(C.c_void_p(fr.data_ptr()), 10, 2, 160, 120, C.c_void_p(out.data_ptr()), None) == -1  # stride < frame
     prm = _lib.FarnebackParams(3, 0.5, 0, 15, 3, 5, 1.2, 4)       # OPTFLOW_USE_INITIAL_FLOW: not implemented (the op has no flow input)
     h = C.c_void_p()
@@ -616,18 +630,26 @@ def test_gray_entry_point_and_pointer_table_paths(torch, ops):
 
 
 def test_farneback_more_pairs_than_one_pointer_table(torch, ops):
-    """70 pairs in one call: the per-level launches are chunked at the 64-entry pointer table;
-    frames shared by two chunks must get their pyramid / polynomial expansion exactly once."""
-    h, w, n = 64, 96, 70
-    clip = synth.textured_clip(21, n + 1, h, w, max_shift=1.5)
-    of = ops.OpticalFlow(w, h, max_batch=n)
-    out = of.execute(dev(torch, clip)).cpu().numpy()
-    of1 = ops.OpticalFlow(w, h, max_batch=1)
-    for i in (0, 31, 63, 64, 69):
-        single = of1.execute(dev(torch, clip[i:i + 2])).cpu().numpy()[0]
-        assert np.array_equal(out[i], single), i
-        check_flow(out[i], o_flow(clip[i], clip[i + 1]), i)
-    of.close(); of1.close()
+    """More than 64 pairs in one call: the chain launches are chunked at the 64-entry pointer table and
+    the pyramid / polynomial expansion is launched in slices of 65 frames on the second lane; every pair
+    must equal its single-pair run, flow and fused histogram.  96x64 (2 scales) and 320x256 (4 scales)
+    both take the two-launch pyramid (pyr_h / pyr_v) for levels 1.. ."""
+    for h, w, n in ((64, 96, 70), (256, 320, 66)):
+        clip = synth.textured_clip(21, n + 1, h, w, max_shift=1.5)
+        fr = dev(torch, clip)
+        of = ops.OpticalFlow(w, h, max_batch=n)
+        out = of.execute(fr).cpu().numpy()
+        flow_h, fh = of.execute_with_histogram(fr)
+        flow_h, fh = flow_h.cpu().numpy(), fh.cpu().numpy()
+        assert np.array_equal(flow_h, out)
+        of1 = ops.OpticalFlow(w, h, max_batch=1)
+        for i in (0, 31, 63, 64, n - 1):
+            single = of1.execute(fr[i:i + 2]).cpu().numpy()[0]
+            assert np.array_equal(out[i], single), (w, h, i)
+            _, single_fh = of1.execute_with_histogram(fr[i:i + 2])
+            assert np.array_equal(fh[i], single_fh.cpu().numpy()[0]), (w, h, i)
+            check_flow(out[i], o_flow(clip[i], clip[i + 1]), (w, h, i))
+        of.close(); of1.close()
 
 
 def test_cuda_graph_replay_equals_direct_launches(torch, ops):
