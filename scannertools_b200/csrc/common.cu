@@ -1,4 +1,4 @@
-// Error reporting and library-level entry points of the C ABI (include/stb.h).
+// Error reporting, device queries and library-level entry points of the C ABI (include/stb.h).
 #include "stb_rt.h"
 
 #include <cstring>
@@ -22,6 +22,27 @@ int cuda_fail(cudaError_t e, const char* what) {
   // cudaErrorNoDevice = 100, cudaErrorInsufficientDriver = 35
   if ((int)e == 100 || (int)e == 35) return STB_ERR_NO_DEVICE;
   return (int)e > 0 ? (int)e : STB_ERR_INVALID;
+}
+
+int current_device() {
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
+  return dev;
+}
+
+int num_sms() {
+#ifdef STB_CPU_EMU
+  return 2;
+#else
+  static int cached[64] = {};
+  const int dev = current_device();
+  if (cached[dev] == 0) {
+    int n = 0;
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) cached[dev] = n;
+    else return 148;
+  }
+  return cached[dev];
+#endif
 }
 
 }  // namespace stb

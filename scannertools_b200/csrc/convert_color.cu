@@ -71,7 +71,7 @@ int stb_color_out_channels(int code) {
 int stb_convert_color_u8(const uint8_t* const* d_src, int n, int width, int height, int code, uint8_t* const* d_dst,
                          stb_stream_t stream) {
   if (n == 0) return STB_OK;
-  if (!d_src || !d_dst || n < 0 || width <= 0 || height <= 0) {
+  if (n < 0 || width <= 0 || height <= 0) {
     set_error("stb_convert_color_u8: invalid argument (n=%d, %dx%d)", n, width, height);
     return STB_ERR_INVALID;
   }
@@ -79,6 +79,8 @@ int stb_convert_color_u8(const uint8_t* const* d_src, int n, int width, int heig
     set_error("stb_convert_color_u8: conversion code %d is not implemented (RGB/BGR2HSV, RGB/BGR2GRAY, RGB<->BGR)", code);
     return STB_ERR_UNSUPPORTED;
   }
+  if (int rc = check_ptr_table(d_src, n, "stb_convert_color_u8", "source frame")) return rc;
+  if (int rc = check_ptr_table(d_dst, n, "stb_convert_color_u8", "destination frame")) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   const unsigned long long npx = (unsigned long long)width * height;
   long long blocks = (long long)((npx + 255) / 256);
@@ -87,15 +89,8 @@ int stb_convert_color_u8(const uint8_t* const* d_src, int n, int width, int heig
     long long cap = (long long)num_sms() * 8 / m;
     if (cap < 1) cap = 1;
     const long long bx = blocks < cap ? blocks : cap;
-    PtrBatch<const uint8_t> a;
-    PtrBatch<uint8_t> b;
-    for (int i = 0; i < kMaxPtrBatch; ++i) { a.p[i] = nullptr; b.p[i] = nullptr; }
-    for (int i = 0; i < m; ++i) {
-      if (!d_src[base + i] || !d_dst[base + i]) { set_error("stb_convert_color_u8: NULL frame %d", base + i); return STB_ERR_INVALID; }
-      a.p[i] = d_src[base + i];
-      b.p[i] = d_dst[base + i];
-    }
-    stb_launch(convert_color_kernel, dim3((unsigned)bx, (unsigned)m), dim3(256), 0, s, a, b, npx, code);
+    stb_launch(convert_color_kernel, dim3((unsigned)bx, (unsigned)m), dim3(256), 0, s, ptr_chunk(d_src, base, m),
+               ptr_chunk(d_dst, base, m), npx, code);
     STB_CHECK_LAUNCH("convert_color_kernel");
   }
   return STB_OK;

@@ -2517,12 +2517,8 @@ static int check_run_args(stb_farneback* h, const uint8_t* const* frames, int n,
   if (!h || !frames || n < 0) { set_error("%s: invalid argument", who); return STB_ERR_INVALID; }
   if (n > h->max_pairs) { set_error("%s: n=%d exceeds max_pairs=%d", who, n, h->max_pairs); return STB_ERR_INVALID; }
   if (n == 0) return STB_OK;
-  if (need_flow && !d_flow) { set_error("%s: d_flow is NULL", who); return STB_ERR_INVALID; }
-  for (int i = 0; i <= n; ++i)
-    if (!frames[i]) { set_error("%s: frame %d is NULL", who, i); return STB_ERR_INVALID; }
-  for (int i = 0; d_flow && i < n; ++i)
-    if (!d_flow[i]) { set_error("%s: d_flow[%d] is NULL", who, i); return STB_ERR_INVALID; }
-  return STB_OK;
+  if (int rc = check_ptr_table(frames, n + 1, who, "frame")) return rc;
+  return d_flow || need_flow ? check_ptr_table(d_flow, n, who, "flow") : STB_OK;
 }
 
 static int ensure_flow0(stb_farneback* h) {
@@ -2544,10 +2540,8 @@ static int to_gray(stb_farneback* h, const uint8_t* const* d_rgb, int F, cudaStr
   if (blocks < 1) blocks = 1;
   for (int base = 0; base < F; base += kMaxPtrBatch) {
     const int mcount = F - base < kMaxPtrBatch ? F - base : kMaxPtrBatch;
-    PtrBatch<const uint8_t> t;
-    for (int i = 0; i < kMaxPtrBatch; ++i) t.p[i] = nullptr;
-    for (int i = 0; i < mcount; ++i) t.p[i] = d_rgb[base + i];
-    stb_launch(gray_kernel, dim3((unsigned)blocks, (unsigned)mcount), dim3(256), 0, s, t, h->gray + (size_t)base * npx, npx);
+    stb_launch(gray_kernel, dim3((unsigned)blocks, (unsigned)mcount), dim3(256), 0, s, ptr_chunk(d_rgb, base, mcount),
+               h->gray + (size_t)base * npx, npx);
     STB_CHECK_LAUNCH("gray_kernel");
   }
   return STB_OK;

@@ -14,16 +14,6 @@
 
 namespace stb {
 
-struct PtrAddrU8 {
-  PtrBatch<const uint8_t> t;
-  __device__ __forceinline__ const uint8_t* operator()(unsigned i) const { return t.p[i]; }
-};
-struct StrideAddrU8 {
-  const uint8_t* base;
-  unsigned long long stride;
-  __device__ __forceinline__ const uint8_t* operator()(unsigned i) const { return base + (unsigned long long)i * stride; }
-};
-
 // -------------------------------------------------------------------------------------------
 // RGB histogram, 16 bins/channel.  The packed RGB24 frame is a flat byte stream: byte at
 // offset a belongs to channel a % 3 and falls in bin (byte >> 4).
@@ -234,18 +224,6 @@ shot_scores_kernel(const int32_t* __restrict__ hist, int n, const int32_t* __res
 // History: one packed-16-bit table per warp (64 KB, 3 blocks / SM, 0.32 of HBM) -> one per 4 warps
 // (0.35) -> this form, with the ~11-instruction packed-counter update gone.
 // -------------------------------------------------------------------------------------------
-struct PtrAddrF32 {
-  PtrBatch<const float> t;
-  __device__ __forceinline__ const float* operator()(unsigned i) const { return t.p[i]; }
-};
-struct StrideAddrF32 {
-  const float* base;
-  unsigned long long stride;  // bytes
-  __device__ __forceinline__ const float* operator()(unsigned i) const {
-    return reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(base) + (unsigned long long)i * stride);
-  }
-};
-
 constexpr int kFlowHistThreads = 256;
 // rows: 64 magnitude bins, one trash row, 64 angle bins, one trash row.  A dropped value (bin outside 0..63)
 // is clamped onto the trash row, so the update needs no predicate: ptxas turns a predicated shared RED into
@@ -355,51 +333,19 @@ frame_diff_kernel(const uint8_t* __restrict__ prev, const uint8_t* __restrict__ 
 // -------------------------------------------------------------------------------------------
 // host side
 // -------------------------------------------------------------------------------------------
-int current_device() {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) dev = 0;
-  return dev;
-}
-
-int num_sms() {
-#ifdef STB_CPU_EMU
-  return 2;
-#else
-  static int cached[64] = {};
-  const int dev = current_device();
-  if (cached[dev] == 0) {
-    int n = 0;
-    if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) cached[dev] = n;
-    else return 148;
-  }
-  return cached[dev];
-#endif
-}
-
 template <class Addr>
 static int launch_hist(Addr addr, int n, unsigned long long nbytes, int32_t* d_out, cudaStream_t s) {
-  static bool attr_done[64] = {};  // per device: the attribute is per (function, device)
-  const int dev = current_device();
-  if (!attr_done[dev]) {
-    STB_CUDA(cudaFuncSetAttribute(hist_rgb16_kernel<Addr>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)kHistSmemBytes));
-    attr_done[dev] = true;
-  }
-  const unsigned long long nvec = nbytes >> 4;
-  // one resident wave (kHistBlocksPerSM blocks/SM) spread over the frames of this launch; never more blocks
-  // than there are 4-vector iterations of work
-  const int wave = num_sms() * kHistBlocksPerSM;
-  // Total blocks: one resident wave split over the frames as evenly as possible
+  if (int rc = set_max_dyn_smem_once<hist_rgb16_kernel<Addr>>(kHistSmemBytes)) return rc;
+  // One resident wave (kHistBlocksPerSM blocks/SM) split over the frames as evenly as possible
   // (some frames get one block more); spilling a handful of blocks into a second wave costs ~25 %,
   // leaving slots empty costs proportionally (n = 32 on 444 slots: 416 blocks 66.8 %, 444 blocks ~71 %).
   // Never more blocks per frame than there are 4-vector iterations of work; with more frames than
   // slots, one block per frame.
+  const unsigned long long nvec = nbytes >> 4;
   const long long max_useful = (long long)((nvec + (unsigned long long)kHistThreads * 4 - 1) / ((unsigned long long)kHistThreads * 4));
-  long long total = wave;
-  if (total < n) total = n;
-  if (max_useful >= 1 && total > max_useful * n) total = max_useful * n;
-  if (total < n) total = n;
-  const unsigned base_blocks = (unsigned)(total / n), rem = (unsigned)(total % n);
+  long long total;
+  unsigned base_blocks, rem;
+  one_wave_split(n, kHistBlocksPerSM, max_useful, &total, &base_blocks, &rem);
   stb_launch(hist_rgb16_kernel<Addr>, dim3((unsigned)total), dim3(kHistThreads), kHistSmemBytes, s, addr, nbytes, d_out,
              base_blocks, rem);
   STB_CHECK_LAUNCH("hist_rgb16_kernel");
@@ -408,19 +354,11 @@ static int launch_hist(Addr addr, int n, unsigned long long nbytes, int32_t* d_o
 
 template <class Addr>
 static int launch_flow_hist(Addr addr, int n, unsigned long long npx, int32_t* d_out, cudaStream_t s) {
-  static bool attr_done[64] = {};
-  const int dev = current_device();
-  if (!attr_done[dev]) {
-    STB_CUDA(cudaFuncSetAttribute(flow_hist_kernel<Addr>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)(kFlowHistSmemWords * sizeof(unsigned))));
-    attr_done[dev] = true;
-  }
-  const int wave = num_sms() * kFlowHistBlocksPerSM;
+  if (int rc = set_max_dyn_smem_once<flow_hist_kernel<Addr>>((int)(kFlowHistSmemWords * sizeof(unsigned)))) return rc;
   const long long max_useful = (long long)((npx / 2 + (unsigned long long)kFlowHistThreads * 2 - 1) / ((unsigned long long)kFlowHistThreads * 2));
-  long long total = wave;                       // one resident wave, split unevenly over the frames
-  if (max_useful >= 1 && total > max_useful * n) total = max_useful * n;
-  if (total < n) total = n;
-  const unsigned base_blocks = (unsigned)(total / n), rem = (unsigned)(total % n);
+  long long total;
+  unsigned base_blocks, rem;
+  one_wave_split(n, kFlowHistBlocksPerSM, max_useful, &total, &base_blocks, &rem);
   stb_launch(flow_hist_kernel<Addr>, dim3((unsigned)total), dim3(kFlowHistThreads), kFlowHistSmemWords * sizeof(unsigned), s,
              addr, npx, d_out, base_blocks, rem);
   STB_CHECK_LAUNCH("flow_hist_kernel");
@@ -432,10 +370,7 @@ int flow_hist_device(const float* const* d_flow, int n, unsigned long long npx, 
   if (zero_out) STB_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * STB_FLOWHIST_INTS * sizeof(int32_t), s));
   for (int base = 0; base < n; base += kMaxPtrBatch) {
     const int m = n - base < kMaxPtrBatch ? n - base : kMaxPtrBatch;
-    PtrAddrF32 a;
-    for (int i = 0; i < m; ++i) a.t.p[i] = d_flow[base + i];
-    for (int i = m; i < kMaxPtrBatch; ++i) a.t.p[i] = nullptr;
-    int rc = launch_flow_hist(a, m, npx, d_out + (size_t)base * STB_FLOWHIST_INTS, s);
+    int rc = launch_flow_hist(PtrAddr<const float>{ptr_chunk(d_flow, base, m)}, m, npx, d_out + (size_t)base * STB_FLOWHIST_INTS, s);
     if (rc) return rc;
   }
   return STB_OK;
@@ -449,32 +384,20 @@ extern "C" {
 
 int stb_hist_rgb16(const uint8_t* const* d_frames, int n, int width, int height, int32_t* d_out, stb_stream_t stream) {
   if (n == 0) return STB_OK;
-  if (!d_frames || !d_out || n < 0 || width <= 0 || height <= 0) {
+  if (!d_out || n < 0 || width <= 0 || height <= 0) {
     set_error("stb_hist_rgb16: invalid argument (n=%d, %dx%d)", n, width, height);
     return STB_ERR_INVALID;
   }
-  cudaStream_t s = (cudaStream_t)stream;
+  if (int rc = check_ptr_table(d_frames, n, "stb_hist_rgb16", "frame")) return rc;
   const unsigned long long nbytes = 3ull * (unsigned long long)width * (unsigned long long)height;
-  for (int i = 0; i < n; ++i)
-    if (!d_frames[i]) { set_error("stb_hist_rgb16: frame %d is NULL", i); return STB_ERR_INVALID; }
-  if (n > kMaxPtrBatch) {
-    // frames carved out of one buffer at a constant stride (a decoder batch / block buffer) need no
-    // pointer table at all: one launch covers the whole batch
-    const ptrdiff_t stride = d_frames[1] - d_frames[0];
-    bool uniform = stride > 0 && (unsigned long long)stride >= nbytes;
-    for (int i = 2; uniform && i < n; ++i) uniform = (d_frames[i] - d_frames[i - 1]) == stride;
-    if (uniform) return stb_hist_rgb16_strided(d_frames[0], (size_t)stride, n, width, height, d_out, stream);
-  }
+  size_t stride = 0;
+  if (uniform_stride(d_frames, n, nbytes, &stride))
+    return stb_hist_rgb16_strided(d_frames[0], stride, n, width, height, d_out, stream);
+  cudaStream_t s = (cudaStream_t)stream;
   STB_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * STB_HIST_INTS * sizeof(int32_t), s));
   for (int base = 0; base < n; base += kMaxPtrBatch) {
     const int m = n - base < kMaxPtrBatch ? n - base : kMaxPtrBatch;
-    PtrAddrU8 a;
-    for (int i = 0; i < m; ++i) {
-      if (!d_frames[base + i]) { set_error("stb_hist_rgb16: frame %d is NULL", base + i); return STB_ERR_INVALID; }
-      a.t.p[i] = d_frames[base + i];
-    }
-    for (int i = m; i < kMaxPtrBatch; ++i) a.t.p[i] = nullptr;
-    int rc = launch_hist(a, m, nbytes, d_out + (size_t)base * STB_HIST_INTS, s);
+    int rc = launch_hist(PtrAddr<const uint8_t>{ptr_chunk(d_frames, base, m)}, m, nbytes, d_out + (size_t)base * STB_HIST_INTS, s);
     if (rc) return rc;
   }
   return STB_OK;
@@ -490,9 +413,9 @@ int stb_hist_rgb16_strided(const uint8_t* d_base, size_t stride_bytes, int n, in
   }
   cudaStream_t s = (cudaStream_t)stream;
   STB_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * STB_HIST_INTS * sizeof(int32_t), s));
-  for (int base = 0; base < n; base += 32768) {
-    const int m = n - base < 32768 ? n - base : 32768;
-    StrideAddrU8 a{d_base + (size_t)base * stride_bytes, (unsigned long long)stride_bytes};
+  for (int base = 0; base < n; base += kMaxStridedFrames) {
+    const int m = n - base < kMaxStridedFrames ? n - base : kMaxStridedFrames;
+    StrideAddr<const uint8_t> a{d_base + (size_t)base * stride_bytes, (unsigned long long)stride_bytes};
     int rc = launch_hist(a, m, nbytes, d_out + (size_t)base * STB_HIST_INTS, s);
     if (rc) return rc;
   }
@@ -514,12 +437,11 @@ int stb_shot_scores(const int32_t* d_hist, int n, const int32_t* d_prev_hist, in
 
 int stb_flow_hist(const float* const* d_flow, int n, int width, int height, int32_t* d_out, stb_stream_t stream) {
   if (n == 0) return STB_OK;
-  if (!d_flow || !d_out || n < 0 || width <= 0 || height <= 0) {
+  if (!d_out || n < 0 || width <= 0 || height <= 0) {
     set_error("stb_flow_hist: invalid argument (n=%d, %dx%d)", n, width, height);
     return STB_ERR_INVALID;
   }
-  for (int i = 0; i < n; ++i)
-    if (!d_flow[i]) { set_error("stb_flow_hist: flow %d is NULL", i); return STB_ERR_INVALID; }
+  if (int rc = check_ptr_table(d_flow, n, "stb_flow_hist", "flow")) return rc;
   return flow_hist_device(d_flow, n, (unsigned long long)width * (unsigned long long)height, d_out, (cudaStream_t)stream, true);
 }
 
@@ -533,10 +455,10 @@ int stb_flow_hist_strided(const float* d_base, size_t stride_bytes, int n, int w
   }
   cudaStream_t s = (cudaStream_t)stream;
   STB_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * STB_FLOWHIST_INTS * sizeof(int32_t), s));
-  for (int base = 0; base < n; base += 32768) {
-    const int m = n - base < 32768 ? n - base : 32768;
-    StrideAddrF32 a{reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(d_base) + (size_t)base * stride_bytes),
-                    (unsigned long long)stride_bytes};
+  for (int base = 0; base < n; base += kMaxStridedFrames) {
+    const int m = n - base < kMaxStridedFrames ? n - base : kMaxStridedFrames;
+    StrideAddr<const float> a{reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(d_base) + (size_t)base * stride_bytes),
+                              (unsigned long long)stride_bytes};
     int rc = launch_flow_hist(a, m, npx, d_out + (size_t)base * STB_FLOWHIST_INTS, s);
     if (rc) return rc;
   }

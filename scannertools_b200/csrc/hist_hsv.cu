@@ -15,16 +15,6 @@
 
 namespace stb {
 
-struct HsvPtrAddr {
-  PtrBatch<const uint8_t> t;
-  __device__ __forceinline__ const uint8_t* operator()(unsigned i) const { return t.p[i]; }
-};
-struct HsvStrideAddr {
-  const uint8_t* base;
-  unsigned long long stride;
-  __device__ __forceinline__ const uint8_t* operator()(unsigned i) const { return base + (unsigned long long)i * stride; }
-};
-
 constexpr int kHsvThreads = 384;
 constexpr int kHsvPlanes = 12 + 16 + 16;                       // H bins 0..11, S, V
 constexpr int kHsvPlaneS = 12, kHsvPlaneV = 28;
@@ -201,21 +191,14 @@ hist_hsv16_kernel(Addr addr, unsigned long long npx, int32_t* __restrict__ out, 
 
 template <class Addr, bool SWAP>
 static int launch_hist_hsv_t(Addr addr, int n, unsigned long long npx, int32_t* d_out, cudaStream_t s) {
-  static bool attr_done[64] = {};  // per device: the attribute is per (function, device)
-  const int dev = current_device();
-  if (!attr_done[dev]) {
-    STB_CUDA(cudaFuncSetAttribute(hist_hsv16_kernel<Addr, SWAP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)kHsvSmemBytes));
-    attr_done[dev] = true;
-  }
+  if (int rc = set_max_dyn_smem_once<hist_hsv16_kernel<Addr, SWAP>>(kHsvSmemBytes)) return rc;
   // one resident wave (3 blocks/SM) split over the frames as evenly as possible, never more
   // blocks per frame than there are two-group iterations of work
   const unsigned long long ngroups = npx / kHsvGroupPx;
   const long long max_useful = (long long)((ngroups + (unsigned long long)kHsvThreads * 2 - 1) / ((unsigned long long)kHsvThreads * 2));
-  long long total = (long long)num_sms() * 3;
-  if (max_useful >= 1 && total > max_useful * n) total = max_useful * n;
-  if (total < n) total = n;
-  const unsigned base_blocks = (unsigned)(total / n), rem = (unsigned)(total % n);
+  long long total;
+  unsigned base_blocks, rem;
+  one_wave_split(n, 3, max_useful, &total, &base_blocks, &rem);
   stb_launch(hist_hsv16_kernel<Addr, SWAP>, dim3((unsigned)total), dim3(kHsvThreads), kHsvSmemBytes, s, addr, npx, d_out,
              base_blocks, rem);
   STB_CHECK_LAUNCH("hist_hsv16_kernel");
@@ -246,29 +229,22 @@ extern "C" {
 int stb_hist_hsv16(const uint8_t* const* d_frames, int n, int width, int height, int code, int32_t* d_out,
                    stb_stream_t stream) {
   if (n == 0) return STB_OK;
-  if (!d_frames || !d_out || n < 0 || width <= 0 || height <= 0) {
+  if (!d_out || n < 0 || width <= 0 || height <= 0) {
     set_error("stb_hist_hsv16: invalid argument (n=%d, %dx%d)", n, width, height);
     return STB_ERR_INVALID;
   }
   bool swap = false;
   if (int rc = hsv_code_swap(code, "stb_hist_hsv16", &swap)) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
+  if (int rc = check_ptr_table(d_frames, n, "stb_hist_hsv16", "frame")) return rc;
   const unsigned long long npx = (unsigned long long)width * (unsigned long long)height;
-  for (int i = 0; i < n; ++i)
-    if (!d_frames[i]) { set_error("stb_hist_hsv16: frame %d is NULL", i); return STB_ERR_INVALID; }
-  if (n > kMaxPtrBatch) {
-    // frames carved out of one buffer at a constant stride: one launch for the whole batch
-    const ptrdiff_t stride = d_frames[1] - d_frames[0];
-    bool uniform = stride > 0 && (unsigned long long)stride >= 3 * npx;
-    for (int i = 2; uniform && i < n; ++i) uniform = (d_frames[i] - d_frames[i - 1]) == stride;
-    if (uniform) return stb_hist_hsv16_strided(d_frames[0], (size_t)stride, n, width, height, code, d_out, stream);
-  }
+  size_t stride = 0;
+  if (uniform_stride(d_frames, n, 3 * npx, &stride))
+    return stb_hist_hsv16_strided(d_frames[0], stride, n, width, height, code, d_out, stream);
+  cudaStream_t s = (cudaStream_t)stream;
   STB_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * STB_HIST_INTS * sizeof(int32_t), s));
   for (int base = 0; base < n; base += kMaxPtrBatch) {
     const int m = n - base < kMaxPtrBatch ? n - base : kMaxPtrBatch;
-    HsvPtrAddr a;
-    for (int i = 0; i < m; ++i) a.t.p[i] = d_frames[base + i];
-    for (int i = m; i < kMaxPtrBatch; ++i) a.t.p[i] = nullptr;
+    PtrAddr<const uint8_t> a{ptr_chunk(d_frames, base, m)};
     if (int rc = launch_hist_hsv(a, m, npx, swap, d_out + (size_t)base * STB_HIST_INTS, s)) return rc;
   }
   return STB_OK;
@@ -286,9 +262,9 @@ int stb_hist_hsv16_strided(const uint8_t* d_base, size_t stride_bytes, int n, in
   if (int rc = hsv_code_swap(code, "stb_hist_hsv16_strided", &swap)) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   STB_CUDA(cudaMemsetAsync(d_out, 0, (size_t)n * STB_HIST_INTS * sizeof(int32_t), s));
-  for (int base = 0; base < n; base += 32768) {
-    const int m = n - base < 32768 ? n - base : 32768;
-    HsvStrideAddr a{d_base + (size_t)base * stride_bytes, (unsigned long long)stride_bytes};
+  for (int base = 0; base < n; base += kMaxStridedFrames) {
+    const int m = n - base < kMaxStridedFrames ? n - base : kMaxStridedFrames;
+    StrideAddr<const uint8_t> a{d_base + (size_t)base * stride_bytes, (unsigned long long)stride_bytes};
     if (int rc = launch_hist_hsv(a, m, npx, swap, d_out + (size_t)base * STB_HIST_INTS, s)) return rc;
   }
   return STB_OK;

@@ -31,11 +31,6 @@
 
 namespace stb {
 
-struct PtrAddrPairU8 {
-  PtrBatch<const uint8_t> src;
-  PtrBatch<uint8_t> dst;
-};
-
 enum { kInterpLinear = 0, kInterpNearest = 1, kInterpArea = 2, kInterpCubic = 3, kInterpLanczos4 = 4 };
 
 __device__ __forceinline__ int cv_round_f(float v) { return __float2int_rn(v); }
@@ -356,7 +351,7 @@ int stb_resize_bilinear_u8(const uint8_t* const* d_src, int n, int src_w, int sr
 int stb_resize_u8(const uint8_t* const* d_src, int n, int src_w, int src_h, int channels, uint8_t* const* d_dst,
                   int dst_w, int dst_h, int interp, stb_stream_t stream) {
   if (n == 0) return STB_OK;
-  if (!d_src || !d_dst || n < 0 || src_w <= 0 || src_h <= 0 || dst_w <= 0 || dst_h <= 0) {
+  if (n < 0 || src_w <= 0 || src_h <= 0 || dst_w <= 0 || dst_h <= 0) {
     set_error("stb_resize_u8: invalid argument (n=%d, %dx%d -> %dx%d)", n, src_w, src_h, dst_w, dst_h);
     return STB_ERR_INVALID;
   }
@@ -368,6 +363,8 @@ int stb_resize_u8(const uint8_t* const* d_src, int n, int src_w, int src_h, int 
     set_error("stb_resize_u8: interpolation %d is not implemented (INTER_LINEAR, INTER_NEAREST, INTER_AREA, INTER_CUBIC, INTER_LANCZOS4)", interp);
     return STB_ERR_UNSUPPORTED;
   }
+  if (int rc = check_ptr_table(d_src, n, "stb_resize_u8", "source frame")) return rc;
+  if (int rc = check_ptr_table(d_dst, n, "stb_resize_u8", "destination frame")) return rc;
   cudaStream_t s = (cudaStream_t)stream;
   // INTER_CUBIC / INTER_LANCZOS4: tap tables built here, uploaded and released in stream order
   const bool taps = interp == kInterpCubic || interp == kInterpLanczos4;
@@ -406,14 +403,8 @@ int stb_resize_u8(const uint8_t* const* d_src, int n, int src_w, int src_h, int 
   const int area2x = (interp == kInterpLinear && src_w == 2 * dst_w && src_h == 2 * dst_h) ? 1 : 0;
   for (int base = 0; base < n; base += kMaxPtrBatch) {
     const int m = n - base < kMaxPtrBatch ? n - base : kMaxPtrBatch;
-    PtrBatch<const uint8_t> a;
-    PtrBatch<uint8_t> b;
-    for (int i = 0; i < kMaxPtrBatch; ++i) { a.p[i] = nullptr; b.p[i] = nullptr; }
-    for (int i = 0; i < m; ++i) {
-      if (!d_src[base + i] || !d_dst[base + i]) { set_error("stb_resize_u8: NULL frame %d", base + i); return STB_ERR_INVALID; }
-      a.p[i] = d_src[base + i];
-      b.p[i] = d_dst[base + i];
-    }
+    const PtrBatch<const uint8_t> a = ptr_chunk(d_src, base, m);
+    const PtrBatch<uint8_t> b = ptr_chunk(d_dst, base, m);
     const dim3 grid(ceil_div(dst_w, 32), ceil_div(dst_h, 8), m);
     if (taps) {
       if (K == 4) {

@@ -345,6 +345,41 @@ def test_emu_flow_compensated_window_equals_global_gathers(emu, h, w, gen):
         assert np.array_equal(res[0][i], res[1][i]), i
 
 
+@pytest.mark.parametrize('op,side', [('convert_color', 'src'), ('convert_color', 'dst'), ('resize_linear', 'src'),
+                                     ('resize_linear', 'dst'), ('resize_cubic', 'src'), ('resize_cubic', 'dst'),
+                                     ('hist_rgb16', 'src'), ('hist_hsv16', 'src'), ('flow_hist', 'src')])
+def test_emu_null_entry_past_first_pointer_table_is_rejected_before_any_launch(emu, op, side):
+    """A NULL entry at index 65 of a 67-frame batch (in the second 64-entry pointer table) is rejected with
+    STB_ERR_INVALID before anything is enqueued: no output of the batch is written, not even the first chunk's."""
+    n, h, w, bad = 67, 4, 8, 65
+    rng = np.random.default_rng(17)
+    if op == 'flow_hist':
+        src = rng.standard_normal((n, h, w, 2)).astype(np.float32)
+    else:
+        src = rng.integers(0, 256, (n, h, w, 3), dtype=np.uint8)
+    if op.startswith('hist') or op == 'flow_hist':
+        out = np.full((n, 128 if op == 'flow_hist' else 48), -7, np.int32)
+    else:
+        out = np.full((n, 3, 5, 3) if op.startswith('resize') else (n, h, w, 3), 0xA5, np.uint8)
+    srcs = [0 if side == 'src' and i == bad else src[i].ctypes.data for i in range(n)]
+    dsts = [0 if side == 'dst' and i == bad else out[i].ctypes.data for i in range(n)]
+    st, dt = _lib.ptr_table(srcs), _lib.ptr_table(dsts)
+    rgb2hsv = emu.stb_color_code(b'COLOR_RGB2HSV')
+    if op == 'convert_color':
+        rc = emu.stb_convert_color_u8(st, n, w, h, rgb2hsv, dt, None)
+    elif op.startswith('resize'):
+        interp = emu.stb_resize_interp_code(b'INTER_CUBIC' if op == 'resize_cubic' else b'INTER_LINEAR')
+        rc = emu.stb_resize_u8(st, n, w, h, 3, dt, 5, 3, interp, None)
+    elif op == 'hist_rgb16':
+        rc = emu.stb_hist_rgb16(st, n, w, h, P(out), None)
+    elif op == 'hist_hsv16':
+        rc = emu.stb_hist_hsv16(st, n, w, h, rgb2hsv, P(out), None)
+    else:
+        rc = emu.stb_flow_hist(st, n, w, h, P(out), None)
+    assert rc == -1 and b'NULL' in emu.stb_last_error(), (rc, emu.stb_last_error())
+    assert (out == (-7 if out.dtype == np.int32 else 0xA5)).all()
+
+
 def test_emu_flow_histogram_fast_binning_randomised(emu):
     """flow_bins_fast (approximate location + exact path inside the guard bands, magic-number rint / floor, trash
     rows for dropped values) against the restatement on a field that mixes generic vectors, magnitudes on and next

@@ -609,6 +609,63 @@ def test_c_abi_error_behaviour_on_device(torch, ops):
         ops.histogram(torch.zeros((1, 4, 4, 3), dtype=torch.uint8))      # host tensor: not a device frame
 
 
+def test_batched_ops_launch_counts(torch, ops):
+    """Kernel launches per call of the batched entry points: one per 64-entry pointer table, one for a histogram batch
+    whose frames lie at a constant stride, one per 32768 frames of a strided call, none for a rejected table."""
+    import ctypes as C
+    from scannertools_b200 import _lib
+    lib = _lib.load()
+    h, w = 8, 16
+    fs, ffs = h * w * 3, h * w * 8
+    src = torch.randint(0, 256, (150 * fs,), dtype=torch.uint8, device='cuda')
+    dst = torch.zeros(150 * fs, dtype=torch.uint8, device='cuda')
+    flow = torch.randn(150 * h * w * 2, device='cuda')
+    out = torch.zeros((32769, 128), dtype=torch.int32, device='cuda')
+    rgb2hsv = lib.stb_color_code(b'COLOR_RGB2HSV')
+
+    def table(t, size, n, slot, null_at=None):
+        return _lib.ptr_table([0 if i == null_at else t.data_ptr() + slot(i) * size for i in range(n)])
+
+    def run(op, n, slot, null_src=None, null_dst=None):
+        s, d = table(src, fs, n, slot, null_src), table(dst, fs, n, slot, null_dst)
+        o = C.c_void_p(out.data_ptr())
+        l0 = lib.stb_launch_count()
+        if op == 'hist_rgb16':
+            rc = lib.stb_hist_rgb16(s, n, w, h, o, None)
+        elif op == 'hist_hsv16':
+            rc = lib.stb_hist_hsv16(s, n, w, h, rgb2hsv, o, None)
+        elif op == 'flow_hist':
+            rc = lib.stb_flow_hist(table(flow, ffs, n, slot, null_src), n, w, h, o, None)
+        elif op == 'convert_color':
+            rc = lib.stb_convert_color_u8(s, n, w, h, rgb2hsv, d, None)
+        else:
+            rc = lib.stb_resize_u8(s, n, w, h, 3, d, w // 2, h // 2, 0, None)
+        torch.cuda.synchronize()
+        return rc, lib.stb_launch_count() - l0
+
+    def uneven(i):                      # slots at no constant stride
+        return i + i // 7
+
+    for op in ('hist_rgb16', 'hist_hsv16', 'flow_hist', 'convert_color', 'resize'):
+        for n in (1, 64, 65, 130):
+            assert run(op, n, uneven) == (0, (n + 63) // 64), (op, n)
+        assert run(op, 67, uneven, null_src=65) == (-1, 0), op
+        if op in ('convert_color', 'resize'):
+            assert run(op, 67, uneven, null_dst=65) == (-1, 0), op
+    for op in ('hist_rgb16', 'hist_hsv16'):
+        assert run(op, 130, lambda i: i) == (0, 1), op
+    n = 32769                           # 1x1 frames, packed
+    packed, packed_flow = torch.randint(0, 256, (n * 3,), dtype=torch.uint8, device='cuda'), torch.randn(n * 2, device='cuda')
+    px, fl, o = C.c_void_p(packed.data_ptr()), C.c_void_p(packed_flow.data_ptr()), C.c_void_p(out.data_ptr())
+    for call in (lambda: lib.stb_hist_rgb16_strided(px, 3, n, 1, 1, o, None),
+                 lambda: lib.stb_hist_hsv16_strided(px, 3, n, 1, 1, rgb2hsv, o, None),
+                 lambda: lib.stb_flow_hist_strided(fl, 8, n, 1, 1, o, None)):
+        l0 = lib.stb_launch_count()
+        assert call() == 0
+        torch.cuda.synchronize()
+        assert lib.stb_launch_count() - l0 == 2
+
+
 def test_gray_entry_point_and_pointer_table_paths(torch, ops):
     """stb_farneback_run_gray (the cv::FarnebackOpticalFlow::calc contract on gray frames) equals
     the RGB entry point fed the same frames; FlowHistogram through the pointer-table entry point
