@@ -165,13 +165,25 @@ STB_API int stb_resize_u8(const uint8_t* const* d_src, int n, int src_w, int src
                           uint8_t* const* d_dst, int dst_w, int dst_h, int interp, stb_stream_t stream);
 
 /* ---- ConvertColor (SURVEY 8f rank 3) -------------------------------------------------------------
- * Replaces cv::cvtColor on 8-bit frames for the conversions the shipped pipelines use:
- * COLOR_RGB2HSV (scannertools/old/cpp_ops/imgproc.cpp:41, feeding the HSV histogram of
- * old/histograms.py:32-36) plus BGR2HSV, RGB2GRAY, BGR2GRAY, RGB<->BGR of
- * scannertools_cpp/imgproc/convert_color_kernel.cpp:19-25,61; bit-exact with OpenCV's integer
- * paths.  stb_color_code maps the reference's conversion names ("COLOR_RGB2HSV", ...) to codes
- * (-1 = not implemented); stb_color_out_channels gives the output channel count. */
+ * Replaces cv::cvtColor(frame, out, code) on packed 8-bit frames (scannertools_cpp/imgproc/
+ * convert_color_kernel.cpp:270-276; COLOR_RGB2HSV also for old/cpp_ops/imgproc.cpp:41, feeding the HSV
+ * histogram of old/histograms.py:32-36); bit-exact with OpenCV's integer paths on every input.
+ * stb_color_code maps the reference's conversion names to codes, both spellings where OpenCV has an
+ * alias (-1 = not implemented; every code is below 99):
+ *   0 RGB2HSV, 1 BGR2HSV, 2 RGB2GRAY, 3 BGR2GRAY, 4 BGR2RGB = RGB2BGR            (3 -> 3 or 1)
+ *   5 BGR2BGRA = RGB2RGBA, 6 BGR2RGBA = RGB2BGRA                                  (3 -> 4, alpha 255)
+ *   7 BGRA2BGR = RGBA2RGB, 8 RGBA2BGR = BGRA2RGB                                  (4 -> 3)
+ *   9 BGRA2RGBA = RGBA2BGRA                                                       (4 -> 4, alpha kept)
+ *  10 GRAY2BGR = GRAY2RGB, 11 GRAY2BGRA = GRAY2RGBA                               (1 -> 3 / 4, alpha 255)
+ *  12 BGRA2GRAY, 13 RGBA2GRAY                                                     (4 -> 1)
+ *  14 BGR2YCrCb, 15 RGB2YCrCb, 16 YCrCb2BGR, 17 YCrCb2RGB                         (3 -> 3)
+ *  18 BGR2YUV, 19 RGB2YUV, 20 YUV2BGR, 21 YUV2RGB  (packed 4:4:4)                 (3 -> 3)
+ *  22 BGR2HSV_FULL, 23 RGB2HSV_FULL  (H over [0,256))                             (3 -> 3)
+ * (names without their COLOR_ prefix).  stb_color_in_channels / stb_color_out_channels give a code's
+ * channel counts (0 for an unknown code); stb_convert_color_u8 reads in-channel frames and writes
+ * out-channel frames, n of them, width x height pixels each. */
 STB_API int stb_color_code(const char* name);
+STB_API int stb_color_in_channels(int code);
 STB_API int stb_color_out_channels(int code);
 STB_API int stb_convert_color_u8(const uint8_t* const* d_src, int n, int width, int height, int code,
                                  uint8_t* const* d_dst, stb_stream_t stream);

@@ -58,6 +58,8 @@ class ConvertColorKernelGPU : public BatchedKernel {
 
   void validate(Result* result) override { result->CopyFrom(valid_); }
 
+  int code() const { return code_; }
+
   void new_stream(const std::vector<u8>& args) {
     std::string conv;
     if (!parse_conversion(args, &conv)) { RESULT_ERROR(&valid_, "ConvertColor: could not parse ConvertColorArgs"); return; }
@@ -69,9 +71,13 @@ class ConvertColorKernelGPU : public BatchedKernel {
     CU_CHECK(cudaSetDevice(device_.id));
     const Frame* frame = frame_col[0].as_const_frame();
     const i32 input_count = (i32)num_rows(frame_col);
-    if (frame->type != FrameType::U8 || frame->channels() != 3) {
-      // every conversion implemented here (convert_color_kernel.cpp:19-25,61) reads packed 3-channel bytes
-      STB_FATAL("ConvertColor (B200): only 3-channel U8 frames are implemented");
+    const int in_channels = stb_color_in_channels(code_);
+    if (frame->type != FrameType::U8 || frame->channels() != in_channels) {
+      // cv::cvtColor rejects a frame whose depth or channel count does not fit the conversion
+      char msg[256];
+      snprintf(msg, sizeof(msg), "ConvertColor (B200): %s needs %d-channel U8 frames, got %s frames with %d channels",
+               conversion_.c_str(), in_channels, frame->type == FrameType::U8 ? "U8" : "non-U8", (int)frame->channels());
+      STB_FATAL(msg);
     }
     FrameInfo info(frame->height(), frame->width(), stb_color_out_channels(code_), FrameType::U8);
     std::vector<Frame*> output_frames = new_frames(device_, info, input_count);
@@ -88,6 +94,7 @@ class ConvertColorKernelGPU : public BatchedKernel {
 
  private:
   void set_conversion(const std::string& conv) {
+    conversion_ = conv;
     code_ = stb_color_code(conv.c_str());
     if (code_ < 0) RESULT_ERROR(&valid_, "ConvertColor (B200): conversion type %s is not implemented", conv.c_str());
   }
@@ -95,6 +102,7 @@ class ConvertColorKernelGPU : public BatchedKernel {
   DeviceHandle device_;
   cudaStream_t stream_;
   int code_;
+  std::string conversion_;
   Result valid_;
   std::vector<const uint8_t*> src_;
   std::vector<uint8_t*> dst_;
@@ -127,7 +135,7 @@ extern "C" __attribute__((visibility("default"))) int stb_shim_convert_color(con
   k->validate(&r);
   if (!r.success()) return -4;
   DeviceHandle dev{DeviceType::GPU, device_id};
-  FrameInfo info(h, w, 3, FrameType::U8);
+  FrameInfo info(h, w, stb_color_in_channels(k->code()), FrameType::U8);
   std::vector<Frame*> in = new_frames(dev, info, n);
   BatchedElements input(1), output(1);
   for (int i = 0; i < n; ++i) {

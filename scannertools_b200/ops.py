@@ -226,8 +226,18 @@ def resize(frames, width=0, height=0, min=False, preserve_aspect=False, interpol
 
 def convert_color(frames, conversion='COLOR_RGB2HSV', stream=None):
     """ConvertColor op (scannertools_cpp/imgproc/convert_color_kernel.cpp:239-281) / ConvertToHSVCPP
-    (old/cpp_ops/imgproc.cpp:14-48) on uint8 RGB frames; bit-exact with cv::cvtColor.  Implemented:
-    COLOR_RGB2HSV, COLOR_BGR2HSV, COLOR_RGB2GRAY, COLOR_BGR2GRAY, COLOR_BGR2RGB, COLOR_RGB2BGR."""
+    (old/cpp_ops/imgproc.cpp:14-48) on uint8 frames; bit-exact with cv::cvtColor.  `frames` is one
+    [n,H,W,C] / [H,W,C] tensor or a sequence of [H,W,C] tensors, C the conversion's input channel count
+    (1-channel inputs are [n,H,W,1] / [H,W,1]); returns uint8 [n,H,W,out channels].  Implemented
+    (both spellings where OpenCV has an alias):
+      COLOR_RGB2HSV, COLOR_BGR2HSV, COLOR_RGB2HSV_FULL, COLOR_BGR2HSV_FULL (3 -> 3);
+      COLOR_RGB2GRAY, COLOR_BGR2GRAY (3 -> 1); COLOR_RGBA2GRAY, COLOR_BGRA2GRAY (4 -> 1);
+      COLOR_BGR2RGB / RGB2BGR (3 -> 3); COLOR_BGR2BGRA / RGB2RGBA, COLOR_BGR2RGBA / RGB2BGRA (3 -> 4, alpha 255);
+      COLOR_BGRA2BGR / RGBA2RGB, COLOR_RGBA2BGR / BGRA2RGB (4 -> 3); COLOR_BGRA2RGBA / RGBA2BGRA (4 -> 4);
+      COLOR_GRAY2BGR / GRAY2RGB (1 -> 3), COLOR_GRAY2BGRA / GRAY2RGBA (1 -> 4, alpha 255);
+      COLOR_BGR2YCrCb, COLOR_RGB2YCrCb, COLOR_YCrCb2BGR, COLOR_YCrCb2RGB,
+      COLOR_BGR2YUV, COLOR_RGB2YUV, COLOR_YUV2BGR, COLOR_YUV2RGB (packed 4:4:4, 3 -> 3).
+    Any other name raises NotImplementedError; frames with the wrong channel count raise ValueError."""
     torch = _torch()
     lib = _lib.load()
     code = lib.stb_color_code(conversion.encode())
@@ -235,7 +245,7 @@ def convert_color(frames, conversion='COLOR_RGB2HSV', stream=None):
         raise NotImplementedError('ConvertColor: %s is not implemented' % conversion)
     if isinstance(frames, torch.Tensor) and frames.dim() == 3:
         frames = frames.unsqueeze(0)
-    lst, H, W = _frames_list(frames, torch.uint8, 'frames', 3)
+    lst, H, W = _frames_list(frames, torch.uint8, 'frames', lib.stb_color_in_channels(code))
     if not lst:
         raise ValueError('ConvertColor needs at least one frame')
     oc = lib.stb_color_out_channels(code)
