@@ -188,6 +188,21 @@ STB_API int stb_color_out_channels(int code);
 STB_API int stb_convert_color_u8(const uint8_t* const* d_src, int n, int width, int height, int code,
                                  uint8_t* const* d_dst, stb_stream_t stream);
 
+/* ---- Blur ----------------------------------------------------------------------------------------
+ * Replaces the box blur of the reference's BlurKernel (scannertools_cpp/imgproc/blur_kernel_cpu.cpp), which runs
+ * on the CPU only; its BlurArgs.sigma is never read, so this is a box filter, not a Gaussian.  With
+ * k = kernel_size, L = ceil(k/2) - 1 and R = k/2 (an even k puts the extra row and column on the bottom and right),
+ * a pixel with L <= x < width - R and L <= y < height - R gets, for each channel c independently,
+ *   out[y][x][c] = (sum over dy, dx in [-L, R] of in[y+dy][x+dx][c]) / (k*k)
+ * as an unsigned integer sum divided with truncation.  Every other pixel is a copy of the input pixel (the
+ * reference leaves those bytes unwritten), so k = 1 is the identity and a frame smaller than the window is copied
+ * unchanged.  channels: 1, 3 or 4.  n frames of width x height, d_src[i] -> d_dst[i], any alignment.
+ * STB_ERR_INVALID: n < 0, width or height <= 0, other channel counts, kernel_size < 1, or d_dst[i] overlapping
+ * d_src[i] (a blur in place would read half-written rows); aliasing between different frames is the caller's
+ * responsibility.  STB_ERR_UNSUPPORTED: kernel_size > 255.  n == 0 does nothing. */
+STB_API int stb_blur_u8(const uint8_t* const* d_src, int n, int width, int height, int channels, int kernel_size,
+                        uint8_t* const* d_dst, stb_stream_t stream);
+
 /* ---- fused ConvertToHSV -> Histogram (SURVEY 8f rank 3) -------------------------------------------
  * The HSV variant of the shot-detection histogram: scannertools/old/histograms.py:32-36 chains
  * ConvertToHSVCPP (old/cpp_ops/imgproc.cpp:14-48, cv::cvtColor COLOR_RGB2HSV) into the Histogram

@@ -50,6 +50,7 @@ SIGNATURES = {
     'stb_color_in_channels': (C.c_int, [C.c_int]),
     'stb_color_out_channels': (C.c_int, [C.c_int]),
     'stb_convert_color_u8': (C.c_int, [_u8pp, C.c_int, C.c_int, C.c_int, C.c_int, _u8pp, _vp]),
+    'stb_blur_u8': (C.c_int, [_u8pp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _u8pp, _vp]),
     'stb_hist_hsv16': (C.c_int, [_u8pp, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp]),
     'stb_hist_hsv16_strided': (C.c_int, [_vp, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp]),
     'stb_launch_count': (C.c_longlong, []),

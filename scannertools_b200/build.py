@@ -12,7 +12,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 OUT = os.path.join(HERE, 'libscannertools_b200.so')
 OBJ = os.path.join(HERE, 'build')
-SOURCES = ['common.cu', 'hist.cu', 'farneback.cu', 'pipe.cu', 'resize.cu', 'convert_color.cu', 'hist_hsv.cu']
+SOURCES = ['common.cu', 'hist.cu', 'farneback.cu', 'pipe.cu', 'resize.cu', 'convert_color.cu', 'hist_hsv.cu', 'blur.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '-Xcompiler', '-fPIC,-fvisibility=hidden', '-I', os.path.join(ROOT, 'include'), '-I', CSRC]
 
@@ -51,7 +51,8 @@ def build(force=False, verbose=False):
 
 OPS_OUT = os.path.join(HERE, 'libscannertools_imgproc.so')
 OPS_SOURCES = ['histogram_kernel_gpu.cpp', 'optical_flow_kernel_gpu.cpp', 'flow_histogram_kernel_gpu.cpp',
-               'frame_difference_kernel_gpu.cpp', 'resize_kernel_gpu.cpp', 'convert_color_kernel_gpu.cpp', 'compat_runtime.cpp']
+               'frame_difference_kernel_gpu.cpp', 'resize_kernel_gpu.cpp', 'convert_color_kernel_gpu.cpp', 'blur_kernel_gpu.cpp',
+               'compat_runtime.cpp']
 
 
 def build_scanner_ops(force=False, scanner_include=None):
@@ -64,7 +65,8 @@ def build_scanner_ops(force=False, scanner_include=None):
     cuda_home = os.path.dirname(os.path.dirname(nvcc))
     ops_dir = os.path.join(CSRC, 'scanner_ops')
     srcs = [os.path.join(ops_dir, s) for s in OPS_SOURCES if scanner_include is None or s != 'compat_runtime.cpp']
-    deps = srcs + [lib] + [os.path.join(dp, f) for dp, _, fs in os.walk(os.path.join(CSRC, 'scanner_compat')) for f in fs]
+    deps = srcs + [lib] + [os.path.join(ops_dir, f) for f in os.listdir(ops_dir) if f.endswith('.h')]
+    deps += [os.path.join(dp, f) for dp, _, fs in os.walk(os.path.join(CSRC, 'scanner_compat')) for f in fs]
     if not force and not _newer(OPS_OUT, deps):
         return OPS_OUT
     inc = scanner_include or os.path.join(CSRC, 'scanner_compat')

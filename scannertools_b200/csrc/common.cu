@@ -71,3 +71,9 @@ int stb_device_count(void) {
 }
 
 }  // extern "C"
+
+// The CPU emulator library (tests/cuda_emu) is built from a fixed list of translation units; sources added after
+// that list join this one there.  The nvcc build compiles them on their own (build.py SOURCES).
+#ifdef STB_CPU_EMU_BUILD
+#include "blur.cu"
+#endif

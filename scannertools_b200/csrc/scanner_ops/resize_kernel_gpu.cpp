@@ -3,7 +3,7 @@
 // min, preserve_aspect, interpolation; scannertools_imgproc.proto:33-39) arrive through
 // new_stream(args) as a serialized protobuf; target-size rules and the batched output layout
 // are the reference's; cvc::resize (:75-79) is replaced by stb_resize_bilinear_u8.
-// The five scalar fields are decoded with a 30-line wire-format reader so the kernel does not
+// The five fields are decoded with the wire-format reader of proto_wire.h, so the kernel does not
 // need the generated scannertools_imgproc.pb.h.
 #include <string>
 #include <vector>
@@ -12,6 +12,7 @@
 #include "scanner/api/op.h"
 #include "scanner/util/cuda.h"
 #include "scanner/util/memory.h"
+#include "proto_wire.h"
 #include "stb_check.h"
 
 namespace scanner {
@@ -23,48 +24,19 @@ struct ResizeArgsLite {
   std::string interpolation;
 };
 
-bool read_varint(const u8*& p, const u8* end, u64& v) {
-  v = 0;
-  for (int shift = 0; p < end && shift < 64; shift += 7) {
-    const u8 b = *p++;
-    v |= (u64)(b & 0x7f) << shift;
-    if (!(b & 0x80)) return true;
-  }
-  return false;
-}
-
 // protobuf wire format of ResizeArgs: 1 width (varint), 2 height (varint), 3 min (varint),
 // 4 preserve_aspect (varint), 5 interpolation (length-delimited)
 bool parse_resize_args(const std::vector<u8>& buf, ResizeArgsLite* out) {
-  const u8* p = buf.data();
-  const u8* end = p + buf.size();
-  while (p < end) {
-    u64 key;
-    if (!read_varint(p, end, key)) return false;
-    const int field = (int)(key >> 3), wire = (int)(key & 7);
-    if (wire == 0) {
-      u64 v;
-      if (!read_varint(p, end, v)) return false;
-      if (field == 1) out->width = (i32)v;
-      else if (field == 2) out->height = (i32)v;
-      else if (field == 3) out->min = v != 0;
-      else if (field == 4) out->preserve_aspect = v != 0;
-    } else if (wire == 2) {
-      u64 len;
-      if (!read_varint(p, end, len) || len > (u64)(end - p)) return false;
-      if (field == 5) out->interpolation.assign(reinterpret_cast<const char*>(p), (size_t)len);
-      p += len;
-    } else if (wire == 5) {
-      if (end - p < 4) return false;
-      p += 4;
-    } else if (wire == 1) {
-      if (end - p < 8) return false;
-      p += 8;
-    } else {
-      return false;
+  return parse_wire_fields(buf, [out](const WireField& f) {
+    if (f.wire == 0) {
+      if (f.field == 1) out->width = (i32)f.varint;
+      else if (f.field == 2) out->height = (i32)f.varint;
+      else if (f.field == 3) out->min = f.varint != 0;
+      else if (f.field == 4) out->preserve_aspect = f.varint != 0;
+    } else if (f.wire == 2 && f.field == 5) {
+      out->interpolation.assign(reinterpret_cast<const char*>(f.data), f.len);
     }
-  }
-  return true;
+  });
 }
 
 }  // namespace

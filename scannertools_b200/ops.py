@@ -257,6 +257,39 @@ def convert_color(frames, conversion='COLOR_RGB2HSV', stream=None):
     return out
 
 
+def blur(frames, kernel_size, stream=None):
+    """Blur op (scannertools_cpp/imgproc/blur_kernel_cpu.cpp) on uint8 frames with 1, 3 or 4 channels: the
+    reference's k x k box mean (its BlurArgs.sigma is never read), per channel, the window [-L, R] with
+    L = ceil(k/2) - 1 and R = k/2, sum / k^2 truncated.  Pixels whose window leaves the frame are copies of the
+    input (the reference leaves them unwritten).  `frames` is one [n,H,W,C] / [H,W,C] tensor or a sequence of
+    [H,W,C] tensors; returns uint8 [n,H,W,C].  kernel_size < 1 raises ValueError, kernel_size > 255 StbError."""
+    torch = _torch()
+    lib = _lib.load()
+    k = int(kernel_size)
+    if k < 1:
+        raise ValueError('Blur: kernel_size must be >= 1, got %d' % k)
+    if isinstance(frames, torch.Tensor):
+        if frames.dim() == 3:
+            frames = frames.unsqueeze(0)
+        if frames.dim() != 4:
+            raise ValueError('Blur: frames must be [n,H,W,C] or [H,W,C], got shape %s' % (tuple(frames.shape),))
+    else:
+        frames = list(frames)
+    if len(frames) == 0:
+        raise ValueError('Blur needs at least one frame')
+    first = frames[0]
+    if isinstance(first, torch.Tensor) and (first.dim() != 3 or first.shape[-1] not in (1, 3, 4)):
+        raise ValueError('Blur: frames must be [H,W,C] with C in 1, 3, 4, got %s' % (tuple(first.shape),))
+    c = int(first.shape[-1]) if isinstance(first, torch.Tensor) else 0
+    lst, H, W = _frames_list(frames, torch.uint8, 'frames', c)
+    out = torch.empty((len(lst), H, W, c), dtype=torch.uint8, device=lst[0].device)
+    with torch.cuda.device(lst[0].device):
+        st = _lib.ptr_table([f.data_ptr() for f in lst])
+        dt = _lib.ptr_table([out[i].data_ptr() for i in range(len(lst))])
+        _lib.check(lib.stb_blur_u8(st, len(lst), W, H, c, k, dt, _stream_ptr(stream)), lib)
+    return out
+
+
 class OpticalFlow:
     """OpticalFlow op (dense Farneback, the reference's hard-coded parameters).
 

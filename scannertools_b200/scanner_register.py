@@ -7,7 +7,7 @@ Importing this module on a machine with the Scanner engine (`scannerpy`):
     (`@scannerpy.register_python_op(name='ShotBoundaries', batch=BOUNDARY_BATCH)`), its body being
     scannertools_b200.shot_detection.shot_boundaries;
   * registers the kernel library `libscannertools_imgproc.so` (Histogram, OpticalFlow, FlowHistogram,
-    FrameDifference, Resize, ConvertColor GPU kernels) the way scannertools/imgproc/__init__.py:1-3 does
+    FrameDifference, Resize, ConvertColor, Blur GPU kernels) the way scannertools/imgproc/__init__.py:1-3 does
     through scannertools_infra._register_module (scannertools_infra/__init__.py:90-100).
 
 Without `scannerpy` the import fails loudly (there is nothing to register with); the ops themselves
