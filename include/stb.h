@@ -163,6 +163,17 @@ STB_API int stb_resize_bilinear_u8(const uint8_t* const* d_src, int n, int src_w
 STB_API int stb_resize_interp_code(const char* name);
 STB_API int stb_resize_u8(const uint8_t* const* d_src, int n, int src_w, int src_h, int channels,
                           uint8_t* const* d_dst, int dst_w, int dst_h, int interp, stb_stream_t stream);
+/* The same on float32 frames with 1 to 4 channels (an OpticalFlow field is H x W x 2), with the interpolation codes
+ * of stb_resize_interp_code and OpenCV's float arithmetic (cv2.ipp.setUseIPP(False)).  Bit-exact with cv::resize
+ * for INTER_NEAREST, INTER_LINEAR (exact 2x down included) and INTER_AREA up-scaling and integer factors, signed zeros
+ * and infinities included, and for every mode at dst == src size (a copy, as in OpenCV); within
+ * 8 * 2^-23 * max|src| of OpenCV's double-precision result for general INTER_AREA down-scaling, INTER_CUBIC and
+ * INTER_LANCZOS4.  Every frame pointer must be 4-byte aligned.  STB_ERR_UNSUPPORTED: channels outside 1..4, unknown
+ * interp; STB_ERR_INVALID: bad sizes, NULL or misaligned table entries (nothing is enqueued then); n == 0 does
+ * nothing.  INTER_CUBIC / INTER_LANCZOS4 upload their tap tables in stream order, as stb_resize_u8 does: asynchronous,
+ * not graph-capturable. */
+STB_API int stb_resize_f32(const float* const* d_src, int n, int src_w, int src_h, int channels,
+                           float* const* d_dst, int dst_w, int dst_h, int interp, stb_stream_t stream);
 
 /* ---- ConvertColor (SURVEY 8f rank 3) -------------------------------------------------------------
  * Replaces cv::cvtColor(frame, out, code) on packed 8-bit frames (scannertools_cpp/imgproc/

@@ -46,6 +46,7 @@ SIGNATURES = {
     'stb_resize_bilinear_u8': (C.c_int, [_u8pp, C.c_int, C.c_int, C.c_int, C.c_int, _u8pp, C.c_int, C.c_int, _vp]),
     'stb_resize_interp_code': (C.c_int, [C.c_char_p]),
     'stb_resize_u8': (C.c_int, [_u8pp, C.c_int, C.c_int, C.c_int, C.c_int, _u8pp, C.c_int, C.c_int, C.c_int, _vp]),
+    'stb_resize_f32': (C.c_int, [_u8pp, C.c_int, C.c_int, C.c_int, C.c_int, _u8pp, C.c_int, C.c_int, C.c_int, _vp]),
     'stb_color_code': (C.c_int, [C.c_char_p]),
     'stb_color_in_channels': (C.c_int, [C.c_int]),
     'stb_color_out_channels': (C.c_int, [C.c_int]),

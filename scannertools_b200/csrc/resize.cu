@@ -24,7 +24,12 @@
 // elements of a row and the exact integer (sum + 2^21) >> 22 for the scalar tail; Lanczos4 has no vector
 // path for 8-bit frames.  Bit-exact with cv2's own implementation (cv2.ipp.setUseIPP(False)); builds of
 // OpenCV that dispatch 8-bit cubic to IPP differ from OpenCV's own code by one grey level on ~5 % of pixels.
+//
+// Float32 frames with 1 to 4 channels (OpticalFlow's H x W x 2 fields) take the same five paths, chosen by the same
+// host routine (plan_resize), with the same coordinates, area tables and tap tables, and OpenCV's float arithmetic
+// (resize_*_f32_kernel below).
 #include <cmath>
+#include <string>
 #include <vector>
 
 #include "stb_rt.h"
@@ -35,22 +40,17 @@ enum { kInterpLinear = 0, kInterpNearest = 1, kInterpArea = 2, kInterpCubic = 3,
 
 __device__ __forceinline__ int cv_round_f(float v) { return __float2int_rn(v); }
 
-template <int CN>
-__global__ void __launch_bounds__(256)
-resize_linear_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, int sw, int sh, int dw, int dh,
-                        double scale_x, double scale_y, int area2x, int area_mode) {
-  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
-  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
-  if (dx >= dw || dy >= dh) return;
-  const uint8_t* src = srcs.p[blockIdx.z];
-  uint8_t* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
-  if (area2x) {
-    const uint8_t* p = src + ((size_t)(2 * dy) * sw + 2 * dx) * CN;
-    const size_t rs = (size_t)sw * CN;
-#pragma unroll
-    for (int c = 0; c < CN; ++c) dst[c] = (uint8_t)((p[c] + p[CN + c] + p[rs + c] + p[rs + CN + c] + 2) >> 2);
-    return;
-  }
+__device__ __forceinline__ int clamp_index(int i, int n) { return min(max(i, 0), n - 1); }
+
+// Source taps of one linear output pixel, shared by the 8-bit and the float kernels: columns sx, sx1 with fraction
+// fx, rows y0, y1 with fraction fy.
+struct LinearTaps {
+  int sx, sx1, y0, y1;
+  float fx, fy;
+};
+
+__device__ __forceinline__ LinearTaps linear_taps(int dx, int dy, int sw, int sh, int dw, int dh, double scale_x,
+                                                  double scale_y, int area_mode) {
   float fx, fy;
   int sx, sy;
   if (!area_mode) {
@@ -73,12 +73,38 @@ resize_linear_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, in
   }
   if (sx < 0) { fx = 0.f; sx = 0; }
   if (sx >= sw - 1) { fx = 0.f; sx = sw - 1; }
-  const int sx1 = sx + 1 < sw ? sx + 1 : sx;
-  const int a0 = cv_round_f(__fmul_rn(1.f - fx, 2048.f)), a1 = cv_round_f(__fmul_rn(fx, 2048.f));
-  const int b0 = cv_round_f(__fmul_rn(1.f - fy, 2048.f)), b1 = cv_round_f(__fmul_rn(fy, 2048.f));
-  const int y0 = min(max(sy, 0), sh - 1), y1 = min(max(sy + 1, 0), sh - 1);
-  const uint8_t* r0 = src + (size_t)y0 * sw * CN;
-  const uint8_t* r1 = src + (size_t)y1 * sw * CN;
+  LinearTaps t;
+  t.sx = sx;
+  t.sx1 = sx + 1 < sw ? sx + 1 : sx;
+  t.y0 = clamp_index(sy, sh);
+  t.y1 = clamp_index(sy + 1, sh);
+  t.fx = fx;
+  t.fy = fy;
+  return t;
+}
+
+template <int CN>
+__global__ void __launch_bounds__(256)
+resize_linear_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, int sw, int sh, int dw, int dh,
+                        double scale_x, double scale_y, int area2x, int area_mode) {
+  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+  if (dx >= dw || dy >= dh) return;
+  const uint8_t* src = srcs.p[blockIdx.z];
+  uint8_t* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
+  if (area2x) {
+    const uint8_t* p = src + ((size_t)(2 * dy) * sw + 2 * dx) * CN;
+    const size_t rs = (size_t)sw * CN;
+#pragma unroll
+    for (int c = 0; c < CN; ++c) dst[c] = (uint8_t)((p[c] + p[CN + c] + p[rs + c] + p[rs + CN + c] + 2) >> 2);
+    return;
+  }
+  const LinearTaps t = linear_taps(dx, dy, sw, sh, dw, dh, scale_x, scale_y, area_mode);
+  const int sx = t.sx, sx1 = t.sx1;
+  const int a0 = cv_round_f(__fmul_rn(1.f - t.fx, 2048.f)), a1 = cv_round_f(__fmul_rn(t.fx, 2048.f));
+  const int b0 = cv_round_f(__fmul_rn(1.f - t.fy, 2048.f)), b1 = cv_round_f(__fmul_rn(t.fy, 2048.f));
+  const uint8_t* r0 = src + (size_t)t.y0 * sw * CN;
+  const uint8_t* r1 = src + (size_t)t.y1 * sw * CN;
 #pragma unroll
   for (int c = 0; c < CN; ++c) {
     const int h0 = r0[sx * CN + c] * a0 + r0[sx1 * CN + c] * a1;
@@ -89,6 +115,8 @@ resize_linear_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, in
 }
 
 // INTER_NEAREST: sx = min(floor(dx * scale_x), sw - 1) (cv::resizeNN)
+__device__ __forceinline__ int nearest_index(int d, double scale, int sn) { return min(__double2int_rd(d * scale), sn - 1); }
+
 template <int CN>
 __global__ void __launch_bounds__(256)
 resize_nearest_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, int sw, int sh, int dw, int dh,
@@ -96,7 +124,7 @@ resize_nearest_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, i
   const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
   const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
   if (dx >= dw || dy >= dh) return;
-  const int sx = min(__double2int_rd(dx * scale_x), sw - 1), sy = min(__double2int_rd(dy * scale_y), sh - 1);
+  const int sx = nearest_index(dx, scale_x, sw), sy = nearest_index(dy, scale_y, sh);
   const uint8_t* p = srcs.p[blockIdx.z] + ((size_t)sy * sw + sx) * CN;
   uint8_t* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
 #pragma unroll
@@ -214,12 +242,12 @@ resize_taps_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, int 
   for (int k = 0; k < K; ++k) {
     a[k] = xa[dx * K + k];
     b[k] = ya[dy * K + k];
-    cx[k] = min(max(sx0 + k, 0), sw - 1) * CN;
+    cx[k] = clamp_index(sx0 + k, sw) * CN;
   }
   int hsum[K][CN];
 #pragma unroll
   for (int j = 0; j < K; ++j) {
-    const uint8_t* r = src + (size_t)min(max(sy0 + j, 0), sh - 1) * sw * CN;
+    const uint8_t* r = src + (size_t)clamp_index(sy0 + j, sh) * sw * CN;
 #pragma unroll
     for (int c = 0; c < CN; ++c) {
       int h = 0;
@@ -247,6 +275,168 @@ resize_taps_u8_kernel(PtrBatch<const uint8_t> srcs, PtrBatch<uint8_t> dsts, int 
     }
     dst[c] = (uint8_t)min(max(v, 0), 255);
   }
+}
+
+// ---- float32 frames (a flow field is H x W x 2) ----------------------------------------------------------------
+// The same taps as the 8-bit kernels with OpenCV's float arithmetic: every product and sum is rounded on its own
+// (__fmul_rn / __fadd_rn, no FMA contraction) in the order cv::resize's float path uses, and nothing is rounded to
+// an integer.  Frames are 4-byte aligned float arrays read and written one element at a time.
+
+template <int CN>
+__global__ void __launch_bounds__(256)
+resize_nearest_f32_kernel(PtrBatch<const float> srcs, PtrBatch<float> dsts, int sw, int sh, int dw, int dh,
+                          double scale_x, double scale_y) {
+  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+  if (dx >= dw || dy >= dh) return;
+  const int sx = nearest_index(dx, scale_x, sw), sy = nearest_index(dy, scale_y, sh);
+  const float* p = srcs.p[blockIdx.z] + ((size_t)sy * sw + sx) * CN;
+  float* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
+#pragma unroll
+  for (int c = 0; c < CN; ++c) dst[c] = p[c];
+}
+
+// INTER_LINEAR, and INTER_AREA with an up-scaled axis: h = S[sx] * a0 + S[sx1] * a1 per row (a0 = 1 - fx, a1 = fx),
+// out = h0 * b0 + h1 * b1 (HResizeLinear / VResizeLinear in float).  Columns clamped at the right border (sx1 == sx,
+// OpenCV's dx >= xmax) take h = S[sx] * 1 without the neighbour term, so an inf there stays inf, as in OpenCV.
+template <int CN>
+__global__ void __launch_bounds__(256)
+resize_linear_f32_kernel(PtrBatch<const float> srcs, PtrBatch<float> dsts, int sw, int sh, int dw, int dh,
+                         double scale_x, double scale_y, int area_mode) {
+  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+  if (dx >= dw || dy >= dh) return;
+  const LinearTaps t = linear_taps(dx, dy, sw, sh, dw, dh, scale_x, scale_y, area_mode);
+  const float a0 = 1.f - t.fx, a1 = t.fx, b0 = 1.f - t.fy, b1 = t.fy;
+  const float* src = srcs.p[blockIdx.z];
+  const float* r0 = src + (size_t)t.y0 * sw * CN;
+  const float* r1 = src + (size_t)t.y1 * sw * CN;
+  const size_t x0 = (size_t)t.sx * CN, x1 = (size_t)t.sx1 * CN;
+  float* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
+#pragma unroll
+  for (int c = 0; c < CN; ++c) {
+    const float h0 = x1 == x0 ? __fmul_rn(r0[x0 + c], a0) : __fadd_rn(__fmul_rn(r0[x0 + c], a0), __fmul_rn(r0[x1 + c], a1));
+    const float h1 = x1 == x0 ? __fmul_rn(r1[x0 + c], a0) : __fadd_rn(__fmul_rn(r1[x0 + c], a0), __fmul_rn(r1[x1 + c], a1));
+    dst[c] = __fadd_rn(__fmul_rn(h0, b0), __fmul_rn(h1, b1));
+  }
+}
+
+// INTER_AREA with integer factors, and INTER_LINEAR at exactly 2x down (cv::resizeAreaFast_ on float).  With
+// a = (y0, x0), b = (y0, x1), c = (y1, x0), d = (y1, x1) a 2x2 block is ((a + b) + (c + d)) * 0.25 where OpenCV's
+// 4-float vector body runs (every element at 4 channels, the first floor(dw / 4) * 4 pixels of a row at 1 channel)
+// and (0 + (((a + b) + c) + d)) * 0.25 in its scalar code (its sum starts at +0, so a block of -0 gives +0 there).  Other factors: the block in row-major order, summed four
+// elements at a time, (((s0 + s1) + s2) + s3) added to the running sum, the rest one by one, times 1 / area.
+template <int CN>
+__global__ void __launch_bounds__(256)
+resize_area_int_f32_kernel(PtrBatch<const float> srcs, PtrBatch<float> dsts, int sw, int dw, int dh, int isx, int isy) {
+  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+  if (dx >= dw || dy >= dh) return;
+  const size_t rs = (size_t)sw * CN;
+  const float* p = srcs.p[blockIdx.z] + (size_t)dy * isy * rs + (size_t)dx * isx * CN;
+  float* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
+  if (isx == 2 && isy == 2) {
+    const bool vec = CN == 4 || (CN == 1 && dx < (dw & ~3));
+#pragma unroll
+    for (int c = 0; c < CN; ++c) {
+      const float a = p[c], b = p[CN + c], cc = p[rs + c], d = p[rs + CN + c];
+      const float s = vec ? __fadd_rn(__fadd_rn(a, b), __fadd_rn(cc, d))
+                          : __fadd_rn(0.f, __fadd_rn(__fadd_rn(__fadd_rn(a, b), cc), d));
+      dst[c] = __fmul_rn(s, 0.25f);
+    }
+    return;
+  }
+  const int area = isx * isy;
+  const float scale = __fdiv_rn(1.f, (float)area);
+#pragma unroll
+  for (int c = 0; c < CN; ++c) {
+    float sum = 0.f;
+    int i = 0, j = 0;   // block element k = j * isx + i
+    auto next = [&]() {
+      const float v = p[(size_t)j * rs + (size_t)i * CN + c];
+      if (++i == isx) { i = 0; ++j; }
+      return v;
+    };
+    int k = 0;
+    for (; k + 4 <= area; k += 4) {
+      float g = next();
+      g = __fadd_rn(g, next());
+      g = __fadd_rn(g, next());
+      g = __fadd_rn(g, next());
+      sum = __fadd_rn(sum, g);
+    }
+    for (; k < area; ++k) sum = __fadd_rn(sum, next());
+    dst[c] = __fmul_rn(sum, scale);
+  }
+}
+
+// INTER_AREA, general down-scaling: the table order of resize_area_u8_kernel without the final rounding.
+template <int CN>
+__global__ void __launch_bounds__(256)
+resize_area_f32_kernel(PtrBatch<const float> srcs, PtrBatch<float> dsts, int sw, int sh, int dw, int dh,
+                       double scale_x, double scale_y) {
+  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+  if (dx >= dw || dy >= dh) return;
+  const AreaSpan xs = area_span(dx, scale_x, sw), ys = area_span(dy, scale_y, sh);
+  const float* src = srcs.p[blockIdx.z];
+  float* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
+  float sum[CN];
+#pragma unroll
+  for (int c = 0; c < CN; ++c) sum[c] = 0.f;
+  for (int j = 0; j < ys.n; ++j) {
+    const float* r = src + ((size_t)(ys.first + j) * sw + xs.first) * CN;
+    float buf[CN];
+#pragma unroll
+    for (int c = 0; c < CN; ++c) buf[c] = 0.f;
+    for (int i = 0; i < xs.n; ++i) {
+      const float a = xs.alpha(i);
+#pragma unroll
+      for (int c = 0; c < CN; ++c) buf[c] = __fadd_rn(buf[c], __fmul_rn(r[(size_t)i * CN + c], a));
+    }
+    const float beta = ys.alpha(j);
+#pragma unroll
+    for (int c = 0; c < CN; ++c) sum[c] = j == 0 ? __fmul_rn(beta, buf[c]) : __fadd_rn(sum[c], __fmul_rn(beta, buf[c]));
+  }
+#pragma unroll
+  for (int c = 0; c < CN; ++c) dst[c] = sum[c];
+}
+
+// INTER_CUBIC (K = 4) / INTER_LANCZOS4 (K = 8) with the float coefficients of the host tap tables: per source row
+// h = S[x0] * a0 + S[x1] * a1 + ... left to right, then out = h0 * b0 + h1 * b1 + ... top to bottom.
+template <int CN, int K>
+__global__ void __launch_bounds__(256)
+resize_taps_f32_kernel(PtrBatch<const float> srcs, PtrBatch<float> dsts, int sw, int sh, int dw, int dh,
+                       const int* __restrict__ xofs, const float* __restrict__ xa, const int* __restrict__ yofs,
+                       const float* __restrict__ ya) {
+  const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+  const int dy = blockIdx.y * 8 + (threadIdx.x >> 5);
+  if (dx >= dw || dy >= dh) return;
+  const float* src = srcs.p[blockIdx.z];
+  float* dst = dsts.p[blockIdx.z] + ((size_t)dy * dw + dx) * CN;
+  const int sx0 = xofs[dx], sy0 = yofs[dy];
+  float a[K];
+  size_t cx[K];
+#pragma unroll
+  for (int k = 0; k < K; ++k) {
+    a[k] = xa[(size_t)dx * K + k];
+    cx[k] = (size_t)clamp_index(sx0 + k, sw) * CN;
+  }
+  float acc[CN];
+#pragma unroll
+  for (int j = 0; j < K; ++j) {
+    const float* r = src + (size_t)clamp_index(sy0 + j, sh) * sw * CN;
+    const float b = ya[(size_t)dy * K + j];
+#pragma unroll
+    for (int c = 0; c < CN; ++c) {
+      float h = __fmul_rn(r[cx[0] + c], a[0]);
+#pragma unroll
+      for (int k = 1; k < K; ++k) h = __fadd_rn(h, __fmul_rn(r[cx[k] + c], a[k]));
+      acc[c] = j == 0 ? __fmul_rn(h, b) : __fadd_rn(acc[c], __fmul_rn(h, b));
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < CN; ++c) dst[c] = acc[c];
 }
 
 // ---- host side of the tap tables: OpenCV's expressions in OpenCV's precision -------------------------
@@ -283,7 +473,9 @@ static STB_NO_CONTRACT void lanczos4_coeffs(float x, float* c) {       // cv::in
   for (int i = 0; i < 8; ++i) c[i] *= sum;
 }
 
-static STB_NO_CONTRACT void build_taps(int dn, int sn, int K, bool cubic, std::vector<int>& ofs, std::vector<short>& al) {
+// cv::resize's tap tables for INTER_CUBIC / INTER_LANCZOS4: per destination index the first source index (it may lie
+// outside the image) and K float coefficients.
+static STB_NO_CONTRACT void build_taps(int dn, int sn, int K, bool cubic, std::vector<int>& ofs, std::vector<float>& al) {
   const double scale = 1. / ((double)dn / sn);
   ofs.resize(dn);
   al.resize((size_t)dn * K);
@@ -294,12 +486,126 @@ static STB_NO_CONTRACT void build_taps(int dn, int sn, int K, bool cubic, std::v
     float c[8];
     if (cubic) cubic_coeffs(f, c); else lanczos4_coeffs(f, c);
     ofs[d] = s0 - (K / 2 - 1);
-    for (int k = 0; k < K; ++k) {
-      const float v = c[k] * 2048.f;                                   // saturate_cast<short>(cbuf[k] * INTER_RESIZE_COEF_SCALE)
-      const long r = std::lrint(v);                                    // round half to even (default rounding mode)
-      al[(size_t)d * K + k] = (short)(r < -32768 ? -32768 : (r > 32767 ? 32767 : r));
-    }
+    for (int k = 0; k < K; ++k) al[(size_t)d * K + k] = c[k];
   }
+}
+
+// the 8-bit coefficient of a float one: saturate_cast<short>(cbuf[k] * INTER_RESIZE_COEF_SCALE)
+static STB_NO_CONTRACT short tap_coef_u8(float c) {
+  const float v = c * 2048.f;
+  const long r = std::lrint(v);                                        // round half to even (default rounding mode)
+  return (short)(r < -32768 ? -32768 : (r > 32767 ? 32767 : r));
+}
+
+static float tap_coef_f32(float c) { return c; }
+
+// Tap tables on the device, in one allocation [xofs | yofs | xa | ya]; mem is released with cudaFreeAsync.
+template <class Coef>
+struct TapTables {
+  int* mem = nullptr;
+  const int *xofs = nullptr, *yofs = nullptr;
+  const Coef *xa = nullptr, *ya = nullptr;
+};
+
+// Builds the tables on the host and uploads them in stream order.
+template <class Coef>
+static int upload_taps(const char* who, int sw, int sh, int dw, int dh, int K, bool cubic, Coef (*coef)(float),
+                       cudaStream_t s, TapTables<Coef>* t) {
+  std::vector<int> xo, yo;
+  std::vector<float> xa, ya;
+  build_taps(dw, sw, K, cubic, xo, xa);
+  build_taps(dh, sh, K, cubic, yo, ya);
+  const size_t n_int = (size_t)dw + dh, n_coef = xa.size() + ya.size();
+  std::vector<int> host(n_int + (n_coef * sizeof(Coef) + sizeof(int) - 1) / sizeof(int));
+  std::copy(xo.begin(), xo.end(), host.begin());
+  std::copy(yo.begin(), yo.end(), host.begin() + dw);
+  Coef* hc = reinterpret_cast<Coef*>(host.data() + n_int);
+  for (size_t i = 0; i < xa.size(); ++i) hc[i] = coef(xa[i]);
+  for (size_t i = 0; i < ya.size(); ++i) hc[xa.size() + i] = coef(ya[i]);
+  STB_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&t->mem), host.size() * sizeof(int), s));
+  // pageable source: the runtime stages it before returning, so `host` may go out of scope
+  cudaError_t e = cudaMemcpyAsync(t->mem, host.data(), host.size() * sizeof(int), cudaMemcpyHostToDevice, s);
+  if (e != cudaSuccess) {
+    cudaFreeAsync(t->mem, s);
+    t->mem = nullptr;
+    return cuda_fail(e, (std::string(who) + ": tap table upload").c_str());
+  }
+  t->xofs = t->mem;
+  t->yofs = t->mem + dw;
+  t->xa = reinterpret_cast<const Coef*>(t->mem + n_int);
+  t->ya = t->xa + (size_t)dw * K;
+  return STB_OK;
+}
+
+// Which of OpenCV's code paths cv::resize takes for an interpolation code and a pair of sizes.  Both element types
+// select the same way.
+enum ResizePath {
+  kPathNearest,    // INTER_NEAREST, and every mode at dsize == ssize (cv::resize copies the frame; nearest at scale 1
+                   // is that copy, element for element)
+  kPathAreaFast,   // integer factors: INTER_AREA scaled down by whole numbers, INTER_LINEAR by exactly 2
+  kPathArea,       // INTER_AREA scaled down on both axes, other factors
+  kPathLinear,     // INTER_LINEAR, and INTER_AREA with an up-scaled axis (area_coeffs)
+  kPathTaps,       // INTER_CUBIC / INTER_LANCZOS4
+};
+
+struct ResizePlan {
+  ResizePath path;
+  double scale_x, scale_y;   // 1 / (dsize / ssize), as cv::resize forms them
+  int isx, isy;              // kPathAreaFast: the integer factors
+  int area_coeffs;           // kPathLinear: INTER_AREA's coefficients
+};
+
+static ResizePlan plan_resize(int interp, int sw, int sh, int dw, int dh) {
+  ResizePlan p;
+  p.scale_x = 1. / ((double)dw / sw);
+  p.scale_y = 1. / ((double)dh / sh);
+  // cv::resize: iscale = saturate_cast<int>(scale) (round half even); "fast area" when both are integers
+  p.isx = (int)std::nearbyint(p.scale_x);
+  p.isy = (int)std::nearbyint(p.scale_y);
+  const bool int_scale = std::fabs(p.scale_x - p.isx) < 2.220446049250313e-16 && std::fabs(p.scale_y - p.isy) < 2.220446049250313e-16;
+  const bool down = p.scale_x >= 1 && p.scale_y >= 1;
+  p.area_coeffs = interp == kInterpArea ? 1 : 0;
+  if (sw == dw && sh == dh) p.path = kPathNearest;
+  else if (interp == kInterpCubic || interp == kInterpLanczos4) p.path = kPathTaps;
+  else if (interp == kInterpNearest) p.path = kPathNearest;
+  else if (interp == kInterpLinear && sw == 2 * dw && sh == 2 * dh) p.path = kPathAreaFast;
+  else if (interp == kInterpArea && down && int_scale) p.path = kPathAreaFast;
+  else if (interp == kInterpArea && down) p.path = kPathArea;
+  else p.path = kPathLinear;
+  return p;
+}
+
+// The scalar checks of a resize entry point, in the order both report them.
+static int check_resize_args(const char* who, int n, int src_w, int src_h, int dst_w, int dst_h, int channels,
+                             bool channels_ok, const char* channel_list, int interp) {
+  if (n < 0 || src_w <= 0 || src_h <= 0 || dst_w <= 0 || dst_h <= 0) {
+    set_error("%s: invalid argument (n=%d, %dx%d -> %dx%d)", who, n, src_w, src_h, dst_w, dst_h);
+    return STB_ERR_INVALID;
+  }
+  if (!channels_ok) {
+    set_error("%s: %d channels not supported (%s)", who, channels, channel_list);
+    return STB_ERR_UNSUPPORTED;
+  }
+  if (interp < kInterpLinear || interp > kInterpLanczos4) {
+    set_error("%s: interpolation %d is not implemented (INTER_LINEAR, INTER_NEAREST, INTER_AREA, INTER_CUBIC, INTER_LANCZOS4)", who, interp);
+    return STB_ERR_UNSUPPORTED;
+  }
+  return STB_OK;
+}
+
+// float frames are read and written as floats: every entry must be 4-byte aligned
+static int check_float_aligned(const float* const* tab, int n, const char* who, const char* what) {
+  for (int i = 0; i < n; ++i)
+    if (reinterpret_cast<uintptr_t>(tab[i]) % alignof(float)) {
+      set_error("%s: %s %d is not 4-byte aligned", who, what, i);
+      return STB_ERR_INVALID;
+    }
+  return STB_OK;
+}
+
+template <class F>
+static F by_channels(int channels, F c1, F c2, F c3, F c4) {
+  return channels == 1 ? c1 : channels == 2 ? c2 : channels == 3 ? c3 : c4;
 }
 
 }  // namespace stb
@@ -351,80 +657,105 @@ int stb_resize_bilinear_u8(const uint8_t* const* d_src, int n, int src_w, int sr
 int stb_resize_u8(const uint8_t* const* d_src, int n, int src_w, int src_h, int channels, uint8_t* const* d_dst,
                   int dst_w, int dst_h, int interp, stb_stream_t stream) {
   if (n == 0) return STB_OK;
-  if (n < 0 || src_w <= 0 || src_h <= 0 || dst_w <= 0 || dst_h <= 0) {
-    set_error("stb_resize_u8: invalid argument (n=%d, %dx%d -> %dx%d)", n, src_w, src_h, dst_w, dst_h);
-    return STB_ERR_INVALID;
-  }
-  if (channels != 1 && channels != 3 && channels != 4) {
-    set_error("stb_resize_u8: %d channels not supported (1, 3, 4)", channels);
-    return STB_ERR_UNSUPPORTED;
-  }
-  if (interp < kInterpLinear || interp > kInterpLanczos4) {
-    set_error("stb_resize_u8: interpolation %d is not implemented (INTER_LINEAR, INTER_NEAREST, INTER_AREA, INTER_CUBIC, INTER_LANCZOS4)", interp);
-    return STB_ERR_UNSUPPORTED;
-  }
+  if (int rc = check_resize_args("stb_resize_u8", n, src_w, src_h, dst_w, dst_h, channels,
+                                 channels == 1 || channels == 3 || channels == 4, "1, 3, 4", interp))
+    return rc;
   if (int rc = check_ptr_table(d_src, n, "stb_resize_u8", "source frame")) return rc;
   if (int rc = check_ptr_table(d_dst, n, "stb_resize_u8", "destination frame")) return rc;
   cudaStream_t s = (cudaStream_t)stream;
+  const ResizePlan p = plan_resize(interp, src_w, src_h, dst_w, dst_h);
   // INTER_CUBIC / INTER_LANCZOS4: tap tables built here, uploaded and released in stream order
-  const bool taps = interp == kInterpCubic || interp == kInterpLanczos4;
   const int K = interp == kInterpCubic ? 4 : 8;
-  int* d_tab = nullptr;
-  const int *d_xofs = nullptr, *d_yofs = nullptr;
-  const short *d_xa = nullptr, *d_ya = nullptr;
-  if (taps) {
-    std::vector<int> xo, yo;
-    std::vector<short> xa, ya;
-    build_taps(dst_w, src_w, K, interp == kInterpCubic, xo, xa);
-    build_taps(dst_h, src_h, K, interp == kInterpCubic, yo, ya);
-    // one allocation: [xofs | yofs | xa | ya]
-    const size_t n_int = (size_t)dst_w + dst_h, n_short = ((size_t)dst_w + dst_h) * K;
-    std::vector<int> host(n_int + (n_short + 1) / 2);
-    std::copy(xo.begin(), xo.end(), host.begin());
-    std::copy(yo.begin(), yo.end(), host.begin() + dst_w);
-    short* hs = reinterpret_cast<short*>(host.data() + n_int);
-    std::copy(xa.begin(), xa.end(), hs);
-    std::copy(ya.begin(), ya.end(), hs + (size_t)dst_w * K);
-    STB_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&d_tab), host.size() * sizeof(int), s));
-    // pageable source: the runtime stages it before returning, so `host` may go out of scope
-    cudaError_t e = cudaMemcpyAsync(d_tab, host.data(), host.size() * sizeof(int), cudaMemcpyHostToDevice, s);
-    if (e != cudaSuccess) { cudaFreeAsync(d_tab, s); return cuda_fail(e, "stb_resize_u8: tap table upload"); }
-    d_xofs = d_tab;
-    d_yofs = d_tab + dst_w;
-    d_xa = reinterpret_cast<const short*>(d_tab + n_int);
-    d_ya = d_xa + (size_t)dst_w * K;
-  }
+  TapTables<short> t;
+  if (p.path == kPathTaps)
+    if (int rc = upload_taps("stb_resize_u8", src_w, src_h, dst_w, dst_h, K, interp == kInterpCubic, tap_coef_u8, s, &t)) return rc;
   const int vec_elems = interp == kInterpCubic ? (dst_w * channels / 8) * 8 : 0;
-  const double scale_x = 1. / ((double)dst_w / src_w), scale_y = 1. / ((double)dst_h / src_h);
-  // cv::resize: iscale = saturate_cast<int>(scale) (round half even); "fast area" when both are integers
-  const int isx = (int)std::nearbyint(scale_x), isy = (int)std::nearbyint(scale_y);
-  const bool int_scale = std::fabs(scale_x - isx) < 2.220446049250313e-16 && std::fabs(scale_y - isy) < 2.220446049250313e-16;
-  const bool down = scale_x >= 1 && scale_y >= 1;
-  const int area2x = (interp == kInterpLinear && src_w == 2 * dst_w && src_h == 2 * dst_h) ? 1 : 0;
+  const double scale_x = p.scale_x, scale_y = p.scale_y;
   for (int base = 0; base < n; base += kMaxPtrBatch) {
     const int m = n - base < kMaxPtrBatch ? n - base : kMaxPtrBatch;
     const PtrBatch<const uint8_t> a = ptr_chunk(d_src, base, m);
     const PtrBatch<uint8_t> b = ptr_chunk(d_dst, base, m);
     const dim3 grid(ceil_div(dst_w, 32), ceil_div(dst_h, 8), m);
-    if (taps) {
+    if (p.path == kPathTaps) {
       if (K == 4) {
-        if (channels == 3) stb_launch(resize_taps_u8_kernel<3, 4>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, d_xofs, d_xa, d_yofs, d_ya, vec_elems);
-        else if (channels == 1) stb_launch(resize_taps_u8_kernel<1, 4>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, d_xofs, d_xa, d_yofs, d_ya, vec_elems);
-        else stb_launch(resize_taps_u8_kernel<4, 4>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, d_xofs, d_xa, d_yofs, d_ya, vec_elems);
+        if (channels == 3) stb_launch(resize_taps_u8_kernel<3, 4>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya, vec_elems);
+        else if (channels == 1) stb_launch(resize_taps_u8_kernel<1, 4>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya, vec_elems);
+        else stb_launch(resize_taps_u8_kernel<4, 4>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya, vec_elems);
       } else {
-        if (channels == 3) stb_launch(resize_taps_u8_kernel<3, 8>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, d_xofs, d_xa, d_yofs, d_ya, vec_elems);
-        else if (channels == 1) stb_launch(resize_taps_u8_kernel<1, 8>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, d_xofs, d_xa, d_yofs, d_ya, vec_elems);
-        else stb_launch(resize_taps_u8_kernel<4, 8>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, d_xofs, d_xa, d_yofs, d_ya, vec_elems);
+        if (channels == 3) stb_launch(resize_taps_u8_kernel<3, 8>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya, vec_elems);
+        else if (channels == 1) stb_launch(resize_taps_u8_kernel<1, 8>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya, vec_elems);
+        else stb_launch(resize_taps_u8_kernel<4, 8>, grid, dim3(256), 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya, vec_elems);
       }
     }
-    else if (interp == kInterpNearest) STB_RESIZE_DISPATCH(resize_nearest_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y);
-    else if (interp == kInterpArea && down && int_scale) STB_RESIZE_DISPATCH(resize_area_int_u8_kernel, src_w, dst_w, dst_h, isx, isy);
-    else if (interp == kInterpArea && down) STB_RESIZE_DISPATCH(resize_area_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y);
-    else STB_RESIZE_DISPATCH(resize_linear_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y, area2x, interp == kInterpArea ? 1 : 0);
-    if (cudaPeekAtLastError() != cudaSuccess && d_tab) cudaFreeAsync(d_tab, s);
+    else if (p.path == kPathNearest) STB_RESIZE_DISPATCH(resize_nearest_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y);
+    // exact 2x INTER_LINEAR: (a + b + c + d + 2) >> 2 inside the linear kernel
+    else if (p.path == kPathAreaFast && interp == kInterpLinear) STB_RESIZE_DISPATCH(resize_linear_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y, 1, 0);
+    else if (p.path == kPathAreaFast) STB_RESIZE_DISPATCH(resize_area_int_u8_kernel, src_w, dst_w, dst_h, p.isx, p.isy);
+    else if (p.path == kPathArea) STB_RESIZE_DISPATCH(resize_area_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y);
+    else STB_RESIZE_DISPATCH(resize_linear_u8_kernel, src_w, src_h, dst_w, dst_h, scale_x, scale_y, 0, p.area_coeffs);
+    if (cudaPeekAtLastError() != cudaSuccess && t.mem) cudaFreeAsync(t.mem, s);
     STB_CHECK_LAUNCH("resize kernel");
   }
-  if (d_tab) STB_CUDA(cudaFreeAsync(d_tab, s));
+  if (t.mem) STB_CUDA(cudaFreeAsync(t.mem, s));
+  return STB_OK;
+}
+
+int stb_resize_f32(const float* const* d_src, int n, int src_w, int src_h, int channels, float* const* d_dst, int dst_w,
+                   int dst_h, int interp, stb_stream_t stream) {
+  const char* who = "stb_resize_f32";
+  if (n == 0) return STB_OK;
+  if (int rc = check_resize_args(who, n, src_w, src_h, dst_w, dst_h, channels, channels >= 1 && channels <= 4, "1..4", interp))
+    return rc;
+  if (int rc = check_ptr_table(d_src, n, who, "source frame")) return rc;
+  if (int rc = check_ptr_table(d_dst, n, who, "destination frame")) return rc;
+  if (int rc = check_float_aligned(d_src, n, who, "source frame")) return rc;
+  if (int rc = check_float_aligned(d_dst, n, who, "destination frame")) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  const ResizePlan p = plan_resize(interp, src_w, src_h, dst_w, dst_h);
+  TapTables<float> t;
+  if (p.path == kPathTaps)
+    if (int rc = upload_taps(who, src_w, src_h, dst_w, dst_h, interp == kInterpCubic ? 4 : 8, interp == kInterpCubic, tap_coef_f32, s, &t))
+      return rc;
+  const int c = channels;
+  for (int base = 0; base < n; base += kMaxPtrBatch) {
+    const int m = n - base < kMaxPtrBatch ? n - base : kMaxPtrBatch;
+    const PtrBatch<const float> a = ptr_chunk(d_src, base, m);
+    const PtrBatch<float> b = ptr_chunk(d_dst, base, m);
+    const dim3 grid(ceil_div(dst_w, 32), ceil_div(dst_h, 8), m), block(256);
+    switch (p.path) {
+      case kPathNearest:
+        stb_launch(by_channels(c, resize_nearest_f32_kernel<1>, resize_nearest_f32_kernel<2>, resize_nearest_f32_kernel<3>,
+                               resize_nearest_f32_kernel<4>),
+                   grid, block, 0, s, a, b, src_w, src_h, dst_w, dst_h, p.scale_x, p.scale_y);
+        break;
+      case kPathAreaFast:
+        stb_launch(by_channels(c, resize_area_int_f32_kernel<1>, resize_area_int_f32_kernel<2>, resize_area_int_f32_kernel<3>,
+                               resize_area_int_f32_kernel<4>),
+                   grid, block, 0, s, a, b, src_w, dst_w, dst_h, p.isx, p.isy);
+        break;
+      case kPathArea:
+        stb_launch(by_channels(c, resize_area_f32_kernel<1>, resize_area_f32_kernel<2>, resize_area_f32_kernel<3>,
+                               resize_area_f32_kernel<4>),
+                   grid, block, 0, s, a, b, src_w, src_h, dst_w, dst_h, p.scale_x, p.scale_y);
+        break;
+      case kPathLinear:
+        stb_launch(by_channels(c, resize_linear_f32_kernel<1>, resize_linear_f32_kernel<2>, resize_linear_f32_kernel<3>,
+                               resize_linear_f32_kernel<4>),
+                   grid, block, 0, s, a, b, src_w, src_h, dst_w, dst_h, p.scale_x, p.scale_y, p.area_coeffs);
+        break;
+      case kPathTaps:
+        stb_launch(interp == kInterpCubic
+                       ? by_channels(c, resize_taps_f32_kernel<1, 4>, resize_taps_f32_kernel<2, 4>, resize_taps_f32_kernel<3, 4>,
+                                     resize_taps_f32_kernel<4, 4>)
+                       : by_channels(c, resize_taps_f32_kernel<1, 8>, resize_taps_f32_kernel<2, 8>, resize_taps_f32_kernel<3, 8>,
+                                     resize_taps_f32_kernel<4, 8>),
+                   grid, block, 0, s, a, b, src_w, src_h, dst_w, dst_h, t.xofs, t.xa, t.yofs, t.ya);
+        break;
+    }
+    if (cudaPeekAtLastError() != cudaSuccess && t.mem) cudaFreeAsync(t.mem, s);
+    STB_CHECK_LAUNCH("resize kernel");
+  }
+  if (t.mem) STB_CUDA(cudaFreeAsync(t.mem, s));
   return STB_OK;
 }
 

@@ -2,9 +2,11 @@
 // (scannertools_cpp/imgproc/resize_kernel.cpp:22-105): per-stream ResizeArgs (width, height,
 // min, preserve_aspect, interpolation; scannertools_imgproc.proto:33-39) arrive through
 // new_stream(args) as a serialized protobuf; target-size rules and the batched output layout
-// are the reference's; cvc::resize (:75-79) is replaced by stb_resize_bilinear_u8.
+// are the reference's; cvc::resize (:75-79) is replaced by stb_resize_u8 on 8-bit frames and stb_resize_f32 on
+// float frames (OpticalFlow's H x W x 2 fields).
 // The five fields are decoded with the wire-format reader of proto_wire.h, so the kernel does not
 // need the generated scannertools_imgproc.pb.h.
+#include <cstdio>
 #include <string>
 #include <vector>
 
@@ -37,6 +39,10 @@ bool parse_resize_args(const std::vector<u8>& buf, ResizeArgsLite* out) {
       out->interpolation.assign(reinterpret_cast<const char*>(f.data), f.len);
     }
   });
+}
+
+const char* frame_type_name(FrameType t) {
+  return t == FrameType::U8 ? "U8" : t == FrameType::F32 ? "F32" : t == FrameType::F64 ? "F64" : "unknown";
 }
 
 }  // namespace
@@ -87,10 +93,15 @@ class ResizeKernelGPU : public BatchedKernel {
                                 args_.preserve_aspect ? 1 : 0, &target_width, &target_height));
     const i32 input_count = (i32)num_rows(frame_col);
     const int ch = frame->channels();
-    if (frame->type != FrameType::U8 || !(ch == 1 || ch == 3 || ch == 4)) {
-      // resize_kernel.cpp:64 propagates frame->type to cv::resize; only the 8-bit kernels exist here, and an
-      // F32 frame (e.g. a flow field) must not be silently reinterpreted as bytes
-      STB_FATAL("Resize (B200): only U8 frames with 1, 3 or 4 channels are implemented");
+    // resize_kernel.cpp:64 propagates frame->type to cv::resize: 8-bit frames with 1, 3 or 4 channels and float
+    // frames with 1 to 4 (a flow field has 2) have kernels here; anything else must not be reinterpreted as bytes
+    const bool u8 = frame->type == FrameType::U8 && (ch == 1 || ch == 3 || ch == 4);
+    const bool f32 = frame->type == FrameType::F32 && ch >= 1 && ch <= 4;
+    if (!u8 && !f32) {
+      char msg[160];
+      snprintf(msg, sizeof msg, "Resize (B200): %s frames with %d channels are not implemented (U8 with 1, 3 or 4 channels, F32 with 1 to 4)",
+               frame_type_name(frame->type), ch);
+      STB_FATAL(msg);
     }
     FrameInfo info(target_height, target_width, ch, frame->type);
     std::vector<Frame*> output_frames = new_frames(device_, info, input_count);
@@ -100,8 +111,19 @@ class ResizeKernelGPU : public BatchedKernel {
       src_[i] = frame_col[i].as_const_frame()->data;
       dst_[i] = output_frames[i]->data;
     }
-    STB_CHECK(stb_resize_u8(src_.data(), input_count, frame->width(), frame->height(), frame->channels(), dst_.data(),
-                            target_width, target_height, interp_, stream_));
+    if (u8) {
+      STB_CHECK(stb_resize_u8(src_.data(), input_count, frame->width(), frame->height(), ch, dst_.data(), target_width,
+                              target_height, interp_, stream_));
+    } else {
+      std::vector<const float*> fs(input_count);
+      std::vector<float*> fd(input_count);
+      for (i32 i = 0; i < input_count; ++i) {
+        fs[i] = reinterpret_cast<const float*>(src_[i]);
+        fd[i] = reinterpret_cast<float*>(dst_[i]);
+      }
+      STB_CHECK(stb_resize_f32(fs.data(), input_count, frame->width(), frame->height(), ch, fd.data(), target_width,
+                               target_height, interp_, stream_));
+    }
     for (i32 i = 0; i < input_count; ++i) insert_frame(output_columns[0], output_frames[i]);
     CU_CHECK(cudaStreamSynchronize(stream_));
   }
@@ -122,11 +144,10 @@ REGISTER_OP(Resize).frame_input("frame").frame_output("frame");
 
 REGISTER_KERNEL(Resize, ResizeKernelGPU).device(DeviceType::GPU).batch().num_devices(1);
 
-// test harness hook (compat build only): run the kernel with serialized args
+// test harness hooks (compat build only): run the kernel with serialized args on n host frames of w x h x c elements
 #ifdef STB_COMPAT_SHIM
-extern "C" __attribute__((visibility("default"))) int stb_shim_resize(const uint8_t* h_frames, int n, int w, int h, int c,
-                                                                      const uint8_t* args, int args_len, uint8_t* h_out,
-                                                                      int out_capacity, int* out_w, int* out_h, int device_id) {
+static int shim_resize(FrameType type, const void* h_frames, int n, int w, int h, int c, const uint8_t* args, int args_len,
+                       void* h_out, size_t out_capacity, int* out_w, int* out_h, int device_id) {
   KernelConfig cfg;
   cfg.devices.push_back(DeviceHandle{DeviceType::GPU, device_id});
   ResizeKernelGPU k(cfg);
@@ -135,11 +156,12 @@ extern "C" __attribute__((visibility("default"))) int stb_shim_resize(const uint
   k.validate(&r);
   if (!r.success()) return -4;
   DeviceHandle dev{DeviceType::GPU, device_id};
-  FrameInfo info(h, w, c, FrameType::U8);
+  FrameInfo info(h, w, c, type);
   std::vector<Frame*> in = new_frames(dev, info, n);
   BatchedElements input(1), output(1);
   for (int i = 0; i < n; ++i) {
-    CU_CHECK(cudaMemcpy(in[i]->data, h_frames + (size_t)i * info.size(), info.size(), cudaMemcpyHostToDevice));
+    CU_CHECK(cudaMemcpy(in[i]->data, static_cast<const uint8_t*>(h_frames) + (size_t)i * info.size(), info.size(),
+                        cudaMemcpyHostToDevice));
     input[0].push_back(Element(in[i]));
   }
   k.execute(input, output);
@@ -148,14 +170,28 @@ extern "C" __attribute__((visibility("default"))) int stb_shim_resize(const uint
   for (int i = 0; i < n && rc == 0; ++i) {
     Frame* f = output[0][i].as_frame();
     *out_w = f->width(); *out_h = f->height();
-    if ((size_t)(i + 1) * f->size() > (size_t)out_capacity) { rc = -3; break; }
-    CU_CHECK(cudaMemcpy(h_out + (size_t)i * f->size(), f->data, f->size(), cudaMemcpyDeviceToHost));
+    if (f->type != type || (size_t)(i + 1) * f->size() > out_capacity) { rc = -3; break; }
+    CU_CHECK(cudaMemcpy(static_cast<uint8_t*>(h_out) + (size_t)i * f->size(), f->data, f->size(), cudaMemcpyDeviceToHost));
   }
   if (!output[0].empty()) delete_buffer(dev, output[0][0].as_frame()->data);
   for (auto& e : output[0]) delete e.as_frame();
   delete_buffer(dev, in[0]->data);
   for (Frame* f : in) delete f;
   return rc;
+}
+
+extern "C" __attribute__((visibility("default"))) int stb_shim_resize(const uint8_t* h_frames, int n, int w, int h, int c,
+                                                                      const uint8_t* args, int args_len, uint8_t* h_out,
+                                                                      int out_capacity, int* out_w, int* out_h, int device_id) {
+  return shim_resize(FrameType::U8, h_frames, n, w, h, c, args, args_len, h_out, (size_t)out_capacity, out_w, out_h, device_id);
+}
+
+// F32 frames; out_capacity counts floats
+extern "C" __attribute__((visibility("default"))) int stb_shim_resize_f32(const float* h_frames, int n, int w, int h, int c,
+                                                                          const uint8_t* args, int args_len, float* h_out,
+                                                                          int out_capacity, int* out_w, int* out_h, int device_id) {
+  return shim_resize(FrameType::F32, h_frames, n, w, h, c, args, args_len, h_out, (size_t)out_capacity * sizeof(float),
+                     out_w, out_h, device_id);
 }
 #endif  // STB_COMPAT_SHIM
 }  // namespace scanner

@@ -191,11 +191,22 @@ def resize_target(frame_w, frame_h, width=0, height=0, min=False, preserve_aspec
 
 
 def resize(frames, width=0, height=0, min=False, preserve_aspect=False, interpolation='INTER_LINEAR', stream=None):
-    """Resize op (scannertools_cpp/imgproc/resize_kernel.cpp:22-105) on uint8 frames: n frames ->
-    [n, height, width, C], bit-exact with cv::resize for INTER_LINEAR (the default), INTER_NEAREST,
-    INTER_AREA, INTER_LANCZOS4 and INTER_CUBIC (OpenCV's own code path; builds that dispatch 8-bit cubic to
-    IPP differ from it by one grey level on ~5 % of pixels).  The remaining names of the reference's table
-    (:9-20: INTER_MAX, WARP_*, flag values rather than modes) raise NotImplementedError."""
+    """Resize op (scannertools_cpp/imgproc/resize_kernel.cpp:22-105): n frames -> [n, height, width, C] of the
+    input's dtype.  `frames` is one [n,H,W,C] / [H,W,C] tensor or a sequence of [H,W,C] tensors.
+
+    uint8, C in {1, 3, 4}: bit-exact with cv::resize for INTER_LINEAR (the default), INTER_NEAREST, INTER_AREA,
+    INTER_LANCZOS4 and INTER_CUBIC (OpenCV's own code path; builds that dispatch 8-bit cubic to IPP differ from it by
+    one grey level on ~5 % of pixels).
+
+    float32, C in 1..4 (an OpticalFlow field is [H,W,2]), against cv::resize's float code (cv2.ipp.setUseIPP(False)):
+      INTER_NEAREST, INTER_LINEAR (exact 2x down included), INTER_AREA up-scaling and integer factors: bit-exact,
+      signed zeros and infinities included; every mode at the frame's own size: a copy, as in OpenCV;
+      INTER_AREA general down-scaling, INTER_CUBIC, INTER_LANCZOS4: every element within 8 * 2^-23 * max|frame| of
+      OpenCV's double-precision result (general INTER_AREA matches cv2 bit for bit on every size tested).
+    OpenCV builds that send float INTER_LINEAR to IPP differ from OpenCV's own code by up to ~2^-18.6 * max|frame|.
+
+    Other dtypes raise TypeError.  The remaining names of the reference's table (:9-20: INTER_MAX, WARP_*, flag
+    values rather than modes) raise NotImplementedError."""
     torch = _torch()
     lib = _lib.load()
     interp = lib.stb_resize_interp_code((interpolation or '').encode())
@@ -208,19 +219,28 @@ def resize(frames, width=0, height=0, min=False, preserve_aspect=False, interpol
     if isinstance(frames, torch.Tensor) and frames.dim() == 3:
         frames = frames.unsqueeze(0)
     lst = [frames[i] for i in range(frames.shape[0])] if isinstance(frames, torch.Tensor) else list(frames)
-    for f in lst:
-        _require_cuda(f, torch.uint8, 'frames')
     if not lst:
         raise ValueError('Resize needs at least one frame')
+    dtype = lst[0].dtype if isinstance(lst[0], torch.Tensor) else None
+    if dtype not in (torch.uint8, torch.float32):
+        raise TypeError('Resize: frames must be uint8 or float32 CUDA tensors, got %s' % (dtype,))
+    for f in lst:
+        _require_cuda(f, dtype, 'frames')
     H, W, c = lst[0].shape
+    if dtype == torch.float32:
+        if not 1 <= c <= 4:
+            raise ValueError('Resize: float32 frames must have 1 to 4 channels, got %d' % c)
+        if any(tuple(f.shape) != (H, W, c) for f in lst):
+            raise ValueError('Resize: every frame of a batch must have the same shape')
     tw, th = resize_target(W, H, width, height, min, preserve_aspect)
     if tw <= 0 or th <= 0:
         raise ValueError('Resize: target size %dx%d' % (tw, th))
-    out = torch.empty((len(lst), th, tw, c), dtype=torch.uint8, device=lst[0].device)
+    out = torch.empty((len(lst), th, tw, c), dtype=dtype, device=lst[0].device)
+    fn = lib.stb_resize_u8 if dtype == torch.uint8 else lib.stb_resize_f32
     with torch.cuda.device(lst[0].device):
         st = _lib.ptr_table([f.data_ptr() for f in lst])
         dt = _lib.ptr_table([out[i].data_ptr() for i in range(len(lst))])
-        _lib.check(lib.stb_resize_u8(st, len(lst), W, H, c, dt, tw, th, interp, _stream_ptr(stream)), lib)
+        _lib.check(fn(st, len(lst), W, H, c, dt, tw, th, interp, _stream_ptr(stream)), lib)
     return out
 
 
